@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA engine (N > 1: under torchrun)
     python bench.py --impl reference --gpus N ...           # the reference's CPU algorithm (oracle, all host threads)
+    python bench.py ... --dump-outputs DIR                  # also save the last timed step's results as DIR/*.npy
 
 A step = one complete registration job on one synthetic pair (SURVEY section 8d config 2 at N = 1: 1 M-point noisy
 scan vs 1 M-point CAD cloud of the aircraft-panel surface, 5 deg / 2 cm initial offset, gate 1 m): index both clouds,
@@ -303,6 +304,8 @@ def run_ours(args):
         sampler.start()
     times, (res, fit), queries, ms_corr, n_corr_launch = timed(d_tgt, d_src, args.steps, args.warmup)
     launches = eng.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, fit)
     e_times, (e_res, e_fit), e_queries, _, _ = timed(main.h_tgt, main.h_src, args.steps, max(1, args.warmup // 2))
     clocks = sampler.stop() if rank == 0 else None
 
@@ -606,6 +609,19 @@ def run_ours(args):
         sys.exit(3)
 
 
+def dump_outputs(out_dir, res, fit):
+    """What the caller of the timed step receives from its last run, one .npy per value, so that two builds can be
+    compared output for output on the same seeded clouds.  The timings in the result are left out: they differ from
+    run to run."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"transform": np.asarray(res["transform"], np.float32), "fitness": np.float64(fit)}
+    for key in ("converged", "outer_iterations", "inner_iterations", "cost_evaluations", "corr_queries",
+                "corr_pairs_last"):
+        arrays[key] = np.float64(res[key])
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 _JSON_FD = None
 
 
@@ -639,7 +655,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the oracle leg (cpu_baseline and parity_vs_oracle)")
     ap.add_argument("--quick", action="store_true", help="headline + parity only: no config 3 / sweep / FOD rows")
     ap.add_argument("--max-sweep-points", type=int, default=CONFIG3_POINTS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's transform, fitness and iteration counts as "
+                         "DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this repo's engine (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -31,6 +31,13 @@ def test_reference_arm_prints_one_json_line():
     _check(run.stdout, 1)
 
 
+def test_bad_arguments_are_rejected():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        run = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                             timeout=600, cwd=ROOT)
+        assert run.returncode == 2 and run.stdout == "", (extra, run.stderr[-2000:])
+
+
 def test_reference_arm_under_torchrun_rank0_only():
     run = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
                           "--master-addr", "127.0.0.1", "--master-port", "29611", os.path.join(ROOT, "bench.py"), "--impl",

@@ -1,11 +1,13 @@
 """The reference's OWN gtest files, compiled verbatim against the drop-in headers (VERDICT r1 missing #4).
 
-/root/reference/test/test_gicp_alignment.cpp and test_fod_detector.cpp are compiled UNCHANGED with `include/dropin` in
-front of the include path (the header swap of INTEGRATION.md) and tests/cpp/stubs standing in for PCL / Eigen / ROS /
-googletest, and linked against libgicp_b200.so (recipe: oracle/Makefile `ref_tests`; outputs in oracle/_ref/, which is
-git-ignored but travels to the GPU box).  CPU: the two files compile and bind the C ABI.  GPU: the binaries run - the
-reference's three GICPAlignment tests and three FODDetector tests pass on the B200 through the drop-in.
-/root/reference does not exist on the GPU box: nothing here reads it at run time there."""
+The reference (the original leica_point_cloud_processing package) is not part of this repository: these tests run when
+LEICA_REFERENCE_DIR names a checkout of it and skip otherwise.  Its test/test_gicp_alignment.cpp and
+test_fod_detector.cpp are compiled UNCHANGED with `include/dropin` in front of the include path (the header swap of
+INTEGRATION.md) and tests/cpp/stubs standing in for PCL / Eigen / ROS / googletest, and linked against libgicp_b200.so
+(recipe: oracle/Makefile `ref_tests`, which build() runs; outputs in oracle/_ref/, git-ignored).  CPU: the two files
+compile and bind the C ABI.  GPU: the binaries run - the reference's three GICPAlignment tests and three FODDetector
+tests pass on the B200 through the drop-in.  The same cases, restated, run without the reference in test_cpp_shim.py
+and test_segment.py."""
 import json
 import os
 import struct
@@ -14,14 +16,14 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("LEICA_REFERENCE_DIR", "")
 OUT = os.path.join(ROOT, "oracle", "_ref")
 BINARIES = ("ref_test_gicp_alignment", "ref_test_fod_detector")
 
 
 def test_reference_tests_compile_verbatim():
-    if not os.path.isfile(os.path.join(REF, "test", "test_gicp_alignment.cpp")):
-        pytest.skip("/root/reference is not on this machine (the binaries were built where it is)")
+    if not REF or not os.path.isfile(os.path.join(REF, "test", "test_gicp_alignment.cpp")):
+        pytest.skip("LEICA_REFERENCE_DIR does not name a checkout of the reference")
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref_tests"])
     for name, syms in (("ref_test_gicp_alignment", ("gicpb_set_clouds", "gicpb_align", "gicpb_fitness", "gicpb_transform_cloud",
                                                     "gicpb_cloud_resolution", "gicpb_normal_validity")),
@@ -58,7 +60,7 @@ def test_reference_gtests_pass_on_the_gpu(tmp_path, name, n_tests, devices):
     two-rank gicpb_group inside the test's process (both ranks on this box's one GPU, sums through the host)"""
     exe = os.path.join(OUT, name)
     if not os.path.isfile(exe):
-        pytest.skip("oracle/_ref/%s was not built (needs /root/reference at build time)" % name)
+        pytest.skip("oracle/_ref/%s was not built (needs LEICA_REFERENCE_DIR at build time)" % name)
     os.makedirs(tmp_path / "test")
     _write_cube_ply(str(tmp_path / "test" / "cube.ply"))
     env = dict(os.environ, GICPB_STUB_PKG_PATH=str(tmp_path))
