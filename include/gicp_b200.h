@@ -70,7 +70,10 @@ typedef struct gicpb_params {
                                    * search amplifies to ~2e-4 in the final transform (see DESIGN.md section 4) */
   int cost_persistent;            /* 1 (default): the evaluations of one inner solve are commands to ONE resident kernel
                                    * (launched per outer iteration, a third of the pairs parked in shared memory) instead of
-                                   * one launch each; same sums, same bits.  0: one launch per evaluation */
+                                   * one launch each; the same terms, summed in another order (a block owns a
+                                   * contiguous range of pairs): the sums agree with the per-launch kernel's to within
+                                   * 2 n 2^-53 sum|terms|, and repeated evaluations of one state are bit-identical.
+                                   * 0: one launch per evaluation */
 } gicpb_params;
 
 typedef struct gicpb_align_result {
@@ -126,7 +129,10 @@ int gicpb_peer_disable(gicpb_ctx* ctx); /* back to ncclAllReduce (call on every 
  * through the host.  No NCCL is needed.  All clouds are HOST clouds.  A group of one device is a plain context.
  * gicpb_group_ctx(g, r) is a full single-GPU context between group calls (transform, difference, clusters, resolution,
  * normals, ...): used on its own a member never waits for the others.  Clouds set through a member directly are that
- * member's alone; the next gicpb_group_set_clouds replaces them. */
+ * member's alone; the next gicpb_group_set_clouds replaces them.  A member's source index is the group's (that rank's
+ * window of the source): the first call on the member alone that needs the source (gicpb_align, gicpb_fitness,
+ * gicpb_correspondences, gicpb_get_covariances, ...) indexes the whole source and works on all of it, with covariances
+ * computed again for the whole cloud; the next group call goes back to the rank's shard and recomputes them on every member. */
 typedef struct gicpb_group gicpb_group;
 int gicpb_group_create(const int* devices, int n_devices, gicpb_group** out);
 void gicpb_group_destroy(gicpb_group* group);
@@ -267,9 +273,28 @@ int gicpb_get_covariances(gicpb_ctx* ctx, int which, double* cov9);
  * source order (this rank's shard only when sharded): nn_idx (-1 = gated out), d2, maha9 (9 doubles each). */
 int gicpb_correspondences(gicpb_ctx* ctx, const float transform[16], int32_t* nn_idx, float* d2, double* maha9,
                           int64_t* n_pairs);
+/* gicpb_correspondences with the pass chosen: mode 0 = the first pass of a job (unseeded, 1 near probe ring; what
+ * gicpb_correspondences runs), mode 1 = every later pass of gicpb_align (kNearMaxRing rings, each query seeded with the
+ * context's current pairs when use_previous_match is on and those pairs are valid for the same Mahalanobis width). */
+int gicpb_correspondences_pass(gicpb_ctx* ctx, const float transform[16], int mode, int32_t* nn_idx, float* d2,
+                               double* maha9, int64_t* n_pairs);
 /* one evaluation of the objective for the correspondences of the last gicpb_correspondences / align
  * iteration at x = (tx,ty,tz,roll,pitch,yaw): f and g[6] as PCL's OptimizationFunctorWithIndices::fdf */
 int gicpb_cost(gicpb_ctx* ctx, const double x[6], double* f, double g[6]);
+/* n_x evaluations as one inner solve of gicpb_align makes them: x = xs[6 k .. 6 k + 5], f[k], g[6 k .. 6 k + 5], all inside
+ * one evaluation session - one resident kernel when cost_persistent = 1 (and cost_moments = 0), one launch per evaluation
+ * otherwise.  info reports what ran. */
+typedef struct gicpb_cost_session_info {
+  int persistent;              /* 1: the resident kernel evaluated them                                   */
+  int blocks, threads, stages; /* its grid and ring shape (threads x stages)                              */
+  int pairs_per_block;         /* pairs each block owns                                                   */
+  int resident_cap;            /* pairs one block can park in shared memory                               */
+  int resident;                /* pairs each block parks: min(pairs_per_block, resident_cap)              */
+  int epoch_first, epoch_last; /* launch epochs of the session (they differ when the kernel was relaunched) */
+  int64_t launches;            /* kernels launched by the call                                            */
+  int64_t n_pairs;             /* pairs summed by the last evaluation                                     */
+} gicpb_cost_session_info;
+int gicpb_cost_session(gicpb_ctx* ctx, int n_x, const double* xs, double* f, double* g, gicpb_cost_session_info* info);
 /* grid statistics of a cloud index: which = 0 target, 1 source, 2 subtract */
 typedef struct gicpb_grid_info {
   int64_t n_points, n_indexed;

@@ -70,6 +70,22 @@ class GridInfo(ctypes.Structure):
     ]
 
 
+class CostSessionInfo(ctypes.Structure):
+    _fields_ = [
+        ("persistent", ctypes.c_int),
+        ("blocks", ctypes.c_int),
+        ("threads", ctypes.c_int),
+        ("stages", ctypes.c_int),
+        ("pairs_per_block", ctypes.c_int),
+        ("resident_cap", ctypes.c_int),
+        ("resident", ctypes.c_int),
+        ("epoch_first", ctypes.c_int),
+        ("epoch_last", ctypes.c_int),
+        ("launches", ctypes.c_int64),
+        ("n_pairs", ctypes.c_int64),
+    ]
+
+
 class Pc2Layout(ctypes.Structure):
     """gicpb_pc2_layout: where a sensor_msgs/PointCloud2 payload keeps the fields a pcl::PointXYZRGB maps."""
     _fields_ = [
@@ -136,7 +152,11 @@ _SIGNATURES = [
     ("gicpb_knn", ctypes.c_int, [_VOID_P, ctypes.c_int, c_int32_p, c_float_p]),
     ("gicpb_get_covariances", ctypes.c_int, [_VOID_P, ctypes.c_int, c_double_p]),
     ("gicpb_correspondences", ctypes.c_int, [_VOID_P, c_float_p, c_int32_p, c_float_p, c_double_p, c_int64_p]),
+    ("gicpb_correspondences_pass", ctypes.c_int, [_VOID_P, c_float_p, ctypes.c_int, c_int32_p, c_float_p, c_double_p,
+                                                  c_int64_p]),
     ("gicpb_cost", ctypes.c_int, [_VOID_P, c_double_p, c_double_p, c_double_p]),
+    ("gicpb_cost_session", ctypes.c_int, [_VOID_P, ctypes.c_int, c_double_p, c_double_p, c_double_p,
+                                          ctypes.POINTER(CostSessionInfo)]),
     ("gicpb_grid_info_get", ctypes.c_int, [_VOID_P, ctypes.c_int, ctypes.POINTER(GridInfo)]),
     ("gicpb_bench_kernel", ctypes.c_int, [_VOID_P, ctypes.c_int, c_float_p, ctypes.c_int, c_double_p, c_int64_p]),
     ("gicpb_cloud_resolution", ctypes.c_int, [_VOID_P, ctypes.c_int, c_double_p]),
@@ -543,7 +563,9 @@ class Engine:
         self._check(self.lib.gicpb_get_covariances(self.h, which, cov.ctypes.data_as(c_double_p)))
         return cov
 
-    def correspondences(self, T):
+    def correspondences(self, T, seeded=False):
+        """(pairs, idx, d2, maha) of one correspondence pass under T: the first pass of a job, or with seeded=True a later
+        pass (more probe rings, seeded with the current pairs when use_previous_match is on)."""
         Tk, Tp = _T(T)
         n = self.grid_info(1)["n_points"]
         idx = np.empty(n, np.int32)
@@ -551,9 +573,9 @@ class Engine:
         maha = np.empty((n, 3, 3), np.float64)
         maha[:] = np.eye(3)
         pairs = ctypes.c_int64()
-        self._check(self.lib.gicpb_correspondences(self.h, Tp, idx.ctypes.data_as(c_int32_p),
-                                                   d2.ctypes.data_as(c_float_p), maha.ctypes.data_as(c_double_p),
-                                                   ctypes.byref(pairs)))
+        self._check(self.lib.gicpb_correspondences_pass(self.h, Tp, 1 if seeded else 0, idx.ctypes.data_as(c_int32_p),
+                                                        d2.ctypes.data_as(c_float_p), maha.ctypes.data_as(c_double_p),
+                                                        ctypes.byref(pairs)))
         return int(pairs.value), idx, d2, maha
 
     def cost(self, x6):
@@ -563,6 +585,18 @@ class Engine:
         self._check(self.lib.gicpb_cost(self.h, x.ctypes.data_as(c_double_p), ctypes.byref(f),
                                         g.ctypes.data_as(c_double_p)))
         return f.value, g
+
+    def cost_session(self, xs):
+        """f [n], g [n, 6] of the states xs [n, 6] evaluated inside one evaluation session (gicpb_cost_session), and what
+        ran as a dict (persistent, blocks, threads, stages, pairs_per_block, resident_cap, resident, epochs, launches)."""
+        x = np.ascontiguousarray(np.asarray(xs, np.float64).reshape(-1, 6))
+        n = len(x)
+        f = np.empty(n, np.float64)
+        g = np.empty((n, 6), np.float64)
+        info = CostSessionInfo()
+        self._check(self.lib.gicpb_cost_session(self.h, n, x.ctypes.data_as(c_double_p), f.ctypes.data_as(c_double_p),
+                                                g.ctypes.data_as(c_double_p), ctypes.byref(info)))
+        return f, g, {k: int(getattr(info, k)) for k, _ in CostSessionInfo._fields_}
 
     def grid_info(self, which):
         gi = GridInfo()

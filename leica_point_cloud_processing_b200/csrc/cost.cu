@@ -340,7 +340,9 @@ __global__ void __launch_bounds__(kCostThreads) cost_kernel(const float4* __rest
 //     where the other blocks poll (one PCIe reader, not 148); the result goes back through the polled stamp as before;
 //   * block 0 ends the kernel on an EXIT command, or by itself when no command arrived for idle_timeout_ns (a host that
 //     threw an exception, was descheduled, or died): the host notices that the stream has drained and launches again.
-// Sums, order of operations and therefore bits are those of cost_kernel with the same grid.
+// The per-pair arithmetic is cost_kernel's; the order of the sums is not (contiguous ranges per block instead of tiles dealt
+// round-robin over twice as many blocks), so the two kernels agree to the rounding of a reordered sum, not bit for bit.  For
+// one set of pairs and one block shape the order is fixed: the same state gives the same bits in every evaluation.
 template <typename MT, bool kPeer, int kThreads, int kStages>
 __global__ void __launch_bounds__(kThreads, 1)
 cost_persistent_kernel(const float4* __restrict__ src, int lo, int n, const float4* __restrict__ pair_tgt,
@@ -624,7 +626,8 @@ namespace {
 template <typename MT, bool kPeer, int kThreads, int kStages>
 void launch_persistent_v(const float4* src, int lo, int n, const float4* pair_tgt, const void* maha, const CostCommand* hcmd,
                          CostCommand* dcmd, unsigned epoch, double* partials, unsigned* ticket, double* out,
-                         const PeerReduce& pr, unsigned long long idle_ns, int blocks, int smem_optin, cudaStream_t stream) {
+                         const PeerReduce& pr, unsigned long long idle_ns, int blocks, int smem_optin, cudaStream_t stream,
+                         CostPersistentShape* shape) {
   constexpr int kRow = 32 + 6 * (int)sizeof(MT);
   auto kern = cost_persistent_kernel<MT, kPeer, kThreads, kStages>;
   static int static_smem = -1;  // of this instantiation
@@ -637,12 +640,14 @@ void launch_persistent_v(const float4* src, int lo, int n, const float4* pair_tg
   const int budget = smem_optin - static_smem - ring - 1024;  // 1 KB of slack for alignment
   const int per = ((n + blocks - 1) / blocks + 15) & ~15;
   // a multiple of 16 pairs: the row bases of the resident block stay 128-byte aligned
-  const int resident = std::max(0, std::min(per, (budget / kRow) & ~15));
+  const int cap = std::max(0, (budget / kRow) & ~15);
+  const int resident = std::min(per, cap);
   const size_t dyn = (size_t)ring + (size_t)resident * kRow;
   GICPB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
   kern<<<blocks, kThreads, dyn, stream>>>(src, lo, n, pair_tgt, (const MT*)maha, hcmd, dcmd, epoch, partials, ticket, out, pr,
                                           idle_ns, resident);
   GICPB_LAUNCHED();
+  if (shape) *shape = CostPersistentShape{blocks, kThreads, kStages, per, cap, resident};
 }
 
 // block shape of the resident kernel: 512 threads x 2 stages keeps 80 KB in flight per SM and parks 26 % of 1 M pairs;
@@ -662,27 +667,28 @@ int persistent_variant(int n) {
 template <typename MT, bool kPeer>
 void launch_persistent_t(const float4* src, int lo, int n, const float4* pair_tgt, const void* maha, const CostCommand* hcmd,
                          CostCommand* dcmd, unsigned epoch, double* partials, unsigned* ticket, double* out,
-                         const PeerReduce& pr, unsigned long long idle_ns, int blocks, int smem_optin, cudaStream_t stream) {
+                         const PeerReduce& pr, unsigned long long idle_ns, int blocks, int smem_optin, cudaStream_t stream,
+                         CostPersistentShape* shape) {
   switch (persistent_variant(n)) {
     case 1:
       launch_persistent_v<MT, kPeer, 256, 3>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream);
+                                             blocks, smem_optin, stream, shape);
       break;
     case 2:
       launch_persistent_v<MT, kPeer, 256, 2>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream);
+                                             blocks, smem_optin, stream, shape);
       break;
     case 3:
       launch_persistent_v<MT, kPeer, 512, 3>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream);
+                                             blocks, smem_optin, stream, shape);
       break;
     case 4:
       launch_persistent_v<MT, kPeer, 512, 4>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream);
+                                             blocks, smem_optin, stream, shape);
       break;
     default:
       launch_persistent_v<MT, kPeer, 512, 2>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream);
+                                             blocks, smem_optin, stream, shape);
   }
 }
 }  // namespace
@@ -692,23 +698,23 @@ int cost_persistent_blocks(int num_sms) { return num_sms; }
 void launch_cost_persistent(const float4* src, int lo, int n, const float4* pair_tgt, const void* maha, bool maha_fp32,
                             const CostCommand* hcmd_dev, CostCommand* dcmd, unsigned epoch, double* partials, unsigned* ticket,
                             double* out16, const PeerReduce* peer, unsigned long long idle_timeout_ns, int blocks,
-                            int smem_optin, cudaStream_t stream) {
+                            int smem_optin, cudaStream_t stream, CostPersistentShape* shape) {
   PeerReduce pr{};
   if (peer) pr = *peer;
   if (maha_fp32) {
     if (peer)
       launch_persistent_t<float, true>(src, lo, n, pair_tgt, maha, hcmd_dev, dcmd, epoch, partials, ticket, out16, pr,
-                                       idle_timeout_ns, blocks, smem_optin, stream);
+                                       idle_timeout_ns, blocks, smem_optin, stream, shape);
     else
       launch_persistent_t<float, false>(src, lo, n, pair_tgt, maha, hcmd_dev, dcmd, epoch, partials, ticket, out16, pr,
-                                        idle_timeout_ns, blocks, smem_optin, stream);
+                                        idle_timeout_ns, blocks, smem_optin, stream, shape);
   } else {
     if (peer)
       launch_persistent_t<double, true>(src, lo, n, pair_tgt, maha, hcmd_dev, dcmd, epoch, partials, ticket, out16, pr,
-                                        idle_timeout_ns, blocks, smem_optin, stream);
+                                        idle_timeout_ns, blocks, smem_optin, stream, shape);
     else
       launch_persistent_t<double, false>(src, lo, n, pair_tgt, maha, hcmd_dev, dcmd, epoch, partials, ticket, out16, pr,
-                                         idle_timeout_ns, blocks, smem_optin, stream);
+                                         idle_timeout_ns, blocks, smem_optin, stream, shape);
   }
 }
 

@@ -183,10 +183,17 @@ int cost_persistent_blocks(int num_sms);
 // hcmd_dev: device alias of the mapped host command slot of this launch (the host alternates between two slots by epoch,
 // so the EXIT of one launch is never overwritten by the first command of the next); dcmd: one CostCommand in device memory; partials / ticket as
 // launch_cost (blocks rows); out16: mapped host memory of kCostOutDoubles doubles; smem_optin: cudaDevAttrMaxSharedMemoryPerBlockOptin.
+// shape (nullable) receives the block shape the launch took (gicpb_cost_session reports it).
+struct CostPersistentShape {
+  int blocks, threads, stages;
+  int per_block;     // pairs each block owns (a multiple of 16; the last block may own fewer)
+  int resident_cap;  // pairs one block can park in shared memory (a multiple of 16)
+  int resident;      // pairs each full block parks: min(per_block, resident_cap)
+};
 void launch_cost_persistent(const float4* src, int lo, int n, const float4* pair_tgt, const void* maha, bool maha_fp32,
                             const CostCommand* hcmd_dev, CostCommand* dcmd, unsigned epoch, double* partials, unsigned* ticket,
                             double* out16, const PeerReduce* peer, unsigned long long idle_timeout_ns, int blocks,
-                            int smem_optin, cudaStream_t stream);
+                            int smem_optin, cudaStream_t stream, CostPersistentShape* shape = nullptr);
 
 // ---- segment.cu -----------------------------------------------------------------------------------------
 // Euclidean clustering: joins every pair of indexed points of `g` with d2 < r2 (strict) in a union-find over sorted

@@ -247,8 +247,9 @@ def test_align_panel_100k_matches_oracle(engine, oracle):
 @pytest.mark.parametrize("n,fp32", [(5000, 0), (3001, 1), (120_000, 0), (400_001, 1), (400_001, 0)])
 def test_resident_cost_kernel_is_bit_identical(engine, n, fp32):
     """cost_persistent=1 (one resident kernel per inner solve, commands through mapped memory, a part of the pairs parked
-    in shared memory) against cost_persistent=0 (one launch per evaluation): the same sums in the same order, so every
-    evaluation, the trajectory and the final transform are bit-identical - for pair counts below, at and above what the
+    in shared memory) against cost_persistent=0 (one launch per evaluation): the same terms summed in another order, which
+    the float32 transforms absorb, so the trajectory and the final transform are bit-identical - for pair counts below, at
+    and above what the
     resident blocks hold, odd counts, and both Mahalanobis widths."""
     src, tgt, _ = synth.make_pair(n, n)
     out = {}
