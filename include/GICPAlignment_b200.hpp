@@ -155,8 +155,8 @@ inline bool isValidTransform(const Mat4T& tf) {
 // several threads at once need their own (`Context::create()`).
 class Context {
  public:
-  // GICPB_DEVICES=0,1,2,3 (more than one GPU): the registration runs sharded over them inside this process (gicpb_group);
-  // GICPB_DEVICE=n or nothing: one context on that GPU.  get() is always a full single-GPU context (the group's first).
+  // GICPB_DEVICES=0,1,2,3 (more than one GPU): the registration and removeFromCloud's difference run sharded over them
+  // inside this process (gicpb_group); GICPB_DEVICE=n or nothing: one context on that GPU.  get() is always a full single-GPU context (the group's first).
   Context() {
     std::vector<int> devices;
     if (const char* e = std::getenv("GICPB_DEVICES")) {
@@ -213,6 +213,18 @@ class Context {
     else
       check(gicpb_fitness(ctx_, T, max_range, score), "gicpb_fitness");
   }
+  // Filter::removeFromCloud's difference of two host clouds: on every GPU of the group, or on the one context
+  void cloudDifference(const void* input, int64_t n_input, int64_t input_stride, const void* subtract, int64_t n_subtract,
+                       int64_t subtract_stride, double sqr_threshold, uint8_t* mask, int64_t* n_kept) const {
+    if (group_)
+      check_group(gicpb_group_cloud_difference(group_, input, n_input, input_stride, subtract, n_subtract, subtract_stride,
+                                               sqr_threshold, mask, n_kept),
+                  "gicpb_group_cloud_difference");
+    else
+      check(gicpb_cloud_difference(ctx_, input, n_input, input_stride, subtract, n_subtract, subtract_stride, 0,
+                                   sqr_threshold, mask, n_kept),
+            "gicpb_cloud_difference");
+  }
   const char* lastError() const { return group_ ? gicpb_group_last_error(group_) : gicpb_last_error(ctx_); }
   static std::shared_ptr<Context> create() { return std::make_shared<Context>(); }
   // the process-wide context (created on first use, destroyed at exit or by release_shared())
@@ -265,10 +277,9 @@ inline void removeFromCloud(const CloudPtr& input_cloud, const CloudPtr& substra
   std::vector<uint8_t> mask((size_t)n);
   int64_t kept = 0;
   if (n > 0 && !substract_cloud->points.empty()) {
-    shared->check(gicpb_cloud_difference(shared->get(), &input_cloud->points[0].x, n, (int64_t)sizeof(input_cloud->points[0]),
-                                         &substract_cloud->points[0].x, (int64_t)substract_cloud->points.size(),
-                                         (int64_t)sizeof(substract_cloud->points[0]), 0, threshold, mask.data(), &kept),
-                  "gicpb_cloud_difference");
+    shared->cloudDifference(&input_cloud->points[0].x, n, (int64_t)sizeof(input_cloud->points[0]), &substract_cloud->points[0].x,
+                            (int64_t)substract_cloud->points.size(), (int64_t)sizeof(substract_cloud->points[0]), threshold,
+                            mask.data(), &kept);
   }
   CloudT out;
   out.points.reserve((size_t)kept);

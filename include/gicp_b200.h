@@ -145,6 +145,20 @@ int gicpb_group_set_clouds(gicpb_group* group, const void* target, int64_t n_tar
                            const void* source, int64_t n_source, int64_t source_stride_bytes); /* :89-90 */
 int gicpb_group_align(gicpb_group* group, gicpb_align_result* out);                     /* gicp_.align :96,116 */
 int gicpb_group_fitness(gicpb_group* group, const float transform[16], double max_range, double* score); /* :103,123 */
+/* gicpb_cloud_difference over the group (Filter::removeFromCloud, src/Filter.cpp:176-189): host clouds and a host mask,
+ * the same mask and n_kept as one context gives, the same argument errors.  Every member uploads its 1/N of the rows of
+ * both clouds and gets the rest from the other members (GICPB_SHARD_UPLOAD=0: each uploads both clouds whole).  Member r
+ * indexes only its own brick planes of the subtract cloud plus a halo of planes that covers sqrt(sqr_threshold) (the
+ * whole cloud when that halo reaches both ends), answers the finite input points that fall into its own planes, and
+ * writes the mask rows [n_input r / N, n_input (r + 1) / N) from the answers of every member.  A subtract cloud that
+ * cannot be split by planes (too few of them, fewer than 1024 N finite points, a member without points) is indexed
+ * whole by every member, each answering its row slice.  Afterwards a member's subtract index is that window
+ * (gicpb_grid_info_get(ctx, 2) reports it); used on its own, the member indexes the whole subtract cloud again before
+ * gicpb_difference_run, gicpb_cloud_resolution or gicpb_normals on it.  The target and source indexes, covariances and
+ * correspondences of the group are not touched. */
+int gicpb_group_cloud_difference(gicpb_group* group, const void* input, int64_t n_input, int64_t input_stride,
+                                 const void* subtract, int64_t n_subtract, int64_t subtract_stride,
+                                 double sqr_threshold, uint8_t* mask, int64_t* n_kept);
 
 /* ---- clouds: upload once, index on the GPU (replaces setInputTarget / setInputSource and the two FLANN
  *      kd-tree builds, src/GICPAlignment.cpp:89-90; PCL Registration::initCompute[Reciprocal]) ------- */

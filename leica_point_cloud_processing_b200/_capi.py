@@ -181,6 +181,8 @@ _SIGNATURES = [
                                               ctypes.c_int64]),
     ("gicpb_group_align", ctypes.c_int, [_VOID_P, ctypes.POINTER(AlignResult)]),
     ("gicpb_group_fitness", ctypes.c_int, [_VOID_P, c_float_p, ctypes.c_double, c_double_p]),
+    ("gicpb_group_cloud_difference", ctypes.c_int, [_VOID_P, _VOID_P, ctypes.c_int64, ctypes.c_int64, _VOID_P,
+                                                    ctypes.c_int64, ctypes.c_int64, ctypes.c_double, _VOID_P, c_int64_p]),
     ("gicpb_launch_count", ctypes.c_int64, [_VOID_P]),
     ("gicpb_stream", ctypes.c_void_p, [_VOID_P]),
     ("gicpb_last_far_queries", ctypes.c_int64, [_VOID_P]),
@@ -722,3 +724,15 @@ class EngineGroup:
         s = ctypes.c_double()
         self._check(self.lib.gicpb_group_fitness(self.h, Tp, max_range, ctypes.byref(s)))
         return s.value
+
+    def cloud_difference(self, input_cloud, subtract_cloud, sqr_threshold):
+        """Engine.cloud_difference over the group's GPUs: (mask uint8 numpy, kept count).  Host clouds only."""
+        ik, iptr, n, istride, idev = _as_cloud(input_cloud)
+        sk, sptr, ns, sstride, sdev = _as_cloud(subtract_cloud)
+        if idev or sdev:
+            raise ValueError("EngineGroup.cloud_difference takes host clouds")
+        kept = ctypes.c_int64()
+        mask = np.empty(n, np.uint8)
+        self._check(self.lib.gicpb_group_cloud_difference(self.h, iptr, n, istride, sptr, ns, sstride,
+                                                          float(sqr_threshold), mask.ctypes.data, ctypes.byref(kept)))
+        return mask, int(kept.value)

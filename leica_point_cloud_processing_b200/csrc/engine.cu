@@ -225,7 +225,7 @@ struct gicpb_ctx {
     bool sharded = false;    // only this rank's slice of the rows was uploaded: take_prefetch gathers the other ranks'
     bool gathered = false;   // ... unless do_prefetch already did, on the copy stream (one process per GPU)
     int64_t chunk_rows = 0;  // rows per rank in the gathered buffer (the last rank's slice may be shorter, or empty)
-  } prefetch[2];  // 0 target, 1 source
+  } prefetch[4];  // 0 target, 1 source, 2 subtract, 3 difference input (gicpb_group_cloud_difference)
   gicpb_params prm{};
   std::string err;
 
@@ -270,6 +270,9 @@ struct gicpb_ctx {
   DevBuf<unsigned long long> counter;
   DevBuf<unsigned char> far_flags;  // near -> far hand-over (kernels.hpp FarWork)
   DevBuf<unsigned> far_counter;
+  // gicpb_group_cloud_difference: routing of the input rows, this rank's keep bytes in row order, the pieces of its mask slice
+  DevBuf<uint32_t> route_flags, route_pos, route_tmp;
+  DevBuf<unsigned char> keep_full, keep_parts;
 
   NcclApi* nccl = nullptr;
   NcclApi::comm_t comm = nullptr;
@@ -926,13 +929,19 @@ void do_prefetch(gicpb_ctx* c, int which, const void* xyz, int64_t n, int64_t st
   // the index of this cloud may still be in use on the compute stream (its staging buffer is about to be overwritten)
   GICPB_CUDA(cudaEventRecord(c->ev_order, c->stream));
   GICPB_CUDA(cudaStreamWaitEvent(c->copy_stream, c->ev_order, 0));
-  GridIndex& g = which == 0 ? c->tgt : c->src;
+  auto stage = [&](size_t bytes) {  // the cloud's index keeps its staging buffer; the difference input goes to io_a
+    if (which == 3) {
+      c->io_a.reserve(bytes);
+      return c->io_a.get();
+    }
+    return (which == 0 ? c->tgt : which == 1 ? c->src : c->sub).stage(bytes);
+  };
   const unsigned char* src = static_cast<const unsigned char*>(xyz);
   p.sharded = shard_uploads(c);
   if (p.sharded) {
     p.chunk_rows = (n + c->world - 1) / c->world;
     const int64_t lo = std::min<int64_t>(n, (int64_t)c->rank * p.chunk_rows), hi = std::min<int64_t>(n, lo + p.chunk_rows);
-    p.dev = g.stage((size_t)p.chunk_rows * c->world * 12);
+    p.dev = stage((size_t)p.chunk_rows * c->world * 12);
     p.dev_stride = 12;
     if (hi > lo) {
       if (stride == 12 && !HostStager::wants(src + lo * stride, hi - lo, stride))
@@ -942,7 +951,7 @@ void do_prefetch(gicpb_ctx* c, int which, const void* xyz, int64_t n, int64_t st
         c->stager.upload(p.dev + (size_t)lo * 12, src + lo * stride, hi - lo, stride, 12, c->copy_stream);
     }
   } else {
-    p.dev = g.stage((size_t)n * stride);
+    p.dev = stage((size_t)n * stride);
     p.dev_stride = stride;
     if (HostStager::wants(xyz, n, stride)) {  // pageable: packed xyz rows (this call then lasts as long as the gather)
       c->stager.upload(p.dev, src, n, stride, 12, c->copy_stream);
@@ -980,6 +989,15 @@ bool take_prefetch(gicpb_ctx* c, int which, const void* xyz, int64_t n, int64_t 
   GICPB_CUDA(cudaStreamWaitEvent(c->stream, p.done, 0));
   if (p.sharded && !p.gathered) gather_slices(c, which);
   return true;
+}
+
+// keep iff (double)d2 > thr.  With thr_f = largest float <= thr this is d2 > thr_f, i.e. NOT (d2 < next(thr_f)).
+float difference_thr_next(double thr, bool* always_keep) {
+  *always_keep = thr < 0;
+  if (*always_keep) return 0.f;
+  float tf = (float)thr;
+  if ((double)tf > thr) tf = std::nextafterf(tf, -INFINITY);
+  return std::nextafterf(tf, INFINITY);
 }
 
 GridIndex& pick_grid(gicpb_ctx* c, int which) {
@@ -1115,6 +1133,102 @@ int group_run(gicpb_group* g, F fn) {  // fn(rank, ctx) -> status, on one thread
         break;
       }
   return first;
+}
+
+// the argument checks of gicpb_cloud_difference (set_subtract, then run), in its order and with its messages
+void check_difference_args(const void* input, int64_t n_input, int64_t input_stride, const void* subtract,
+                           int64_t n_subtract, int64_t subtract_stride, const uint8_t* mask) {
+  check_cloud_args(subtract, n_subtract, subtract_stride);
+  if (n_subtract > 0x7fffff00LL) throw ArgError("cloud has more than 2^31 points");
+  if (!mask) throw ArgError("null mask");
+  check_cloud_args(input, n_input, input_stride);
+  if (n_input > 0x7fffff00LL) throw ArgError("cloud has more than 2^31 points");
+}
+
+// One rank of gicpb_group_cloud_difference (world > 1, host clouds and mask).  Every rank indexes the subtract planes it owns
+// plus a halo that covers the search radius, answers the finite input rows of its own planes (the other points within the
+// radius of those rows are all in its window) and then assembles the mask of its row slice [lo, hi) from every member's keep
+// bytes.  When the subtract cannot be split by planes every rank indexes all of it and answers its row slice directly.
+// Returns the number of points this rank kept.
+unsigned long long group_difference_rank(gicpb_ctx* c, const void* input, int64_t n, int64_t input_stride,
+                                         const void* subtract, int64_t n_sub, int64_t sub_stride, double thr,
+                                         uint8_t* mask) {
+  bool always_keep = false;
+  const float thr_next = difference_thr_next(thr, &always_keep);
+  const double radius = std::sqrt((double)thr_next);
+  // 1. both clouds: this rank's slice of the rows on the copy stream, the other slices from the other members
+  const void* sub_p = subtract;
+  bool sub_dev = false;
+  const unsigned char* d_in = nullptr;
+  try {
+    if (shard_uploads(c)) {
+      do_prefetch(c, 2, subtract, n_sub, sub_stride);
+      do_prefetch(c, 3, input, n, input_stride);
+    }
+    if (take_prefetch(c, 2, subtract, n_sub, sub_stride, 0)) {
+      sub_p = c->prefetch[2].dev;
+      sub_stride = c->prefetch[2].dev_stride;
+      sub_dev = true;
+    }
+    // 2. the window of the subtract's brick planes
+    c->sub.build(sub_p, n_sub, sub_stride, sub_dev, c->prm.cell_size, c->prm.points_per_cell, c->stream, &c->stager, c->rank,
+                 c->world, std::isfinite(radius) ? radius : INFINITY);
+    if (take_prefetch(c, 3, input, n, input_stride, 0)) {
+      d_in = c->prefetch[3].dev;
+      input_stride = c->prefetch[3].dev_stride;
+    } else {
+      d_in = stage_in(c, c->io_a, input, n, &input_stride, false);
+    }
+  } catch (...) {
+    for (int w : {2, 3})  // a copy started here must not be taken for a later call's clouds
+      if (c->prefetch[w].pending) {
+        c->prefetch[w].pending = false;
+        cudaEventSynchronize(c->prefetch[w].done);
+      }
+    throw;
+  }
+  const int64_t lo = n * c->rank / c->world, hi = n * (c->rank + 1) / c->world, len = hi - lo;
+  const bool routed = c->sub.plane_sharded();
+  c->keep_full.reserve((size_t)n);
+  GICPB_CUDA(cudaMemsetAsync(c->keep_full.get(), 0, (size_t)n, c->stream));
+  GICPB_CUDA(cudaMemsetAsync(c->counter.get(), 0, sizeof(unsigned long long), c->stream));
+  if (routed) {
+    // 3. the rows of this rank's planes, compacted in row order, searched as float4 rows, their keep bytes put back in place
+    c->route_flags.reserve((size_t)n + 1);
+    c->route_pos.reserve((size_t)n + 1);
+    c->route_tmp.reserve(scan_tmp_entries(n + 1));
+    c->queries.reserve((size_t)n);
+    const int64_t n_own = c->sub.owned_queries(d_in, n, input_stride, c->queries.get(), c->route_flags.get(),
+                                                c->route_pos.get(), c->route_tmp.get(), c->stream);
+    c->io_b.reserve((size_t)std::max<int64_t>(n_own, 1));
+    launch_difference(c->sub.view(), reinterpret_cast<const unsigned char*>(c->queries.get()), n_own, 16, thr_next,
+                      always_keep, c->io_b.get(), c->counter.get(), far_work(c, n_own), c->stream);
+    scatter_keep(c->queries.get(), c->io_b.get(), n_own, c->keep_full.get(), c->stream);
+  } else {
+    launch_difference(c->sub.view(), d_in + lo * input_stride, len, input_stride, thr_next, always_keep,
+                      c->keep_full.get() + lo, c->counter.get(), far_work(c, len), c->stream);
+  }
+  unsigned long long kept = 0;
+  GICPB_CUDA(cudaMemcpyAsync(&kept, c->counter.get(), sizeof(kept), cudaMemcpyDeviceToHost, c->stream));
+  GICPB_CUDA(cudaStreamSynchronize(c->stream));
+  // 4. ownership partitions the finite rows: the mask of [lo, hi) is the OR of every member's keep bytes there
+  c->local->barrier();  // every member's keep bytes are complete
+  const unsigned char* slice = c->keep_full.get() + lo;
+  if (routed && len > 0) {
+    c->keep_parts.reserve((size_t)(c->world * len));
+    for (int r = 0; r < c->world; ++r) {
+      const gicpb_ctx* o = c->local->members[(size_t)r];
+      GICPB_CUDA(cudaMemcpyPeerAsync(c->keep_parts.get() + r * len, c->device, o->keep_full.get() + lo, o->device, (size_t)len,
+                                     c->stream));
+    }
+    c->io_b.reserve((size_t)len);
+    or_parts(c->keep_parts.get(), c->world, len, c->io_b.get(), c->stream);
+    slice = c->io_b.get();
+  }
+  GICPB_CUDA(cudaStreamSynchronize(c->stream));
+  c->local->barrier();  // nobody reads another member's keep bytes any more
+  if (len > 0) download_bytes(c, mask + lo, slice, (size_t)len);
+  return kept;
 }
 
 }  // namespace
@@ -1517,6 +1631,7 @@ int gicpb_difference_run(gicpb_ctx* c, const void* input, int64_t n, int64_t str
     check_cloud_args(input, n, stride);
     if (!c->sub.ready()) throw StateError("difference_set_subtract must be called first");
     if (n > 0x7fffff00LL) throw ArgError("cloud has more than 2^31 points");
+    if (c->sub.windowed()) c->sub.widen(c->stream);  // a group member's window of the subtract (gicpb_group_cloud_difference)
     const unsigned char* d_in = stage_in(c, c->io_a, input, n, &stride, on_device != 0);
     unsigned char* d_mask = mask;
     if (!mask_on_device) {
@@ -1524,14 +1639,8 @@ int gicpb_difference_run(gicpb_ctx* c, const void* input, int64_t n, int64_t str
       d_mask = c->io_b.get();
     }
     GICPB_CUDA(cudaMemsetAsync(c->counter.get(), 0, sizeof(unsigned long long), c->stream));
-    // keep iff (double)d2 > thr.  With thr_f = largest float <= thr this is d2 > thr_f, i.e. NOT (d2 < next(thr_f)).
-    bool always_keep = thr < 0;
-    float thr_next = 0.f;
-    if (!always_keep) {
-      float tf = (float)thr;
-      if ((double)tf > thr) tf = std::nextafterf(tf, -INFINITY);
-      thr_next = std::nextafterf(tf, INFINITY);
-    }
+    bool always_keep = false;
+    const float thr_next = difference_thr_next(thr, &always_keep);
     launch_difference(c->sub.view(), d_in, n, stride, thr_next, always_keep, d_mask, c->counter.get(), far_work(c, n),
                       c->stream);
     unsigned long long kept = 0;
@@ -2192,6 +2301,46 @@ int gicpb_group_fitness(gicpb_group* g, const float transform[16], double max_ra
   std::vector<double> sc(g->ctx.size(), 0.0);
   const int rc = group_run(g, [&](int r, gicpb_ctx* c) { return gicpb_fitness(c, transform, max_range, &sc[(size_t)r]); });
   *score = sc[0];
+  return rc;
+}
+
+int gicpb_group_cloud_difference(gicpb_group* g, const void* input, int64_t n_input, int64_t input_stride,
+                                 const void* subtract, int64_t n_subtract, int64_t subtract_stride, double sqr_threshold,
+                                 uint8_t* mask, int64_t* n_kept) {
+  if (!g) return GICPB_E_BADARG;
+  try {
+    check_difference_args(input, n_input, input_stride, subtract, n_subtract, subtract_stride, mask);
+  } catch (const ArgError& e) {
+    g->err = e.what();
+    return GICPB_E_BADARG;
+  }
+  std::vector<int> rcs(g->ctx.size(), GICPB_OK);
+  std::vector<unsigned long long> kept(g->ctx.size(), 0ull);
+  const int rc = group_run(g, [&](int r, gicpb_ctx* c) {
+    if (c->world == 1) {  // a group of one device is a plain context
+      int64_t k = 0;
+      rcs[(size_t)r] = gicpb_cloud_difference(c, input, n_input, input_stride, subtract, n_subtract, subtract_stride, 0,
+                                              sqr_threshold, mask, &k);
+      kept[(size_t)r] = (unsigned long long)k;
+    } else {
+      rcs[(size_t)r] = guarded(c, [&] {
+        kept[(size_t)r] = group_difference_rank(c, input, n_input, input_stride, subtract, n_subtract, subtract_stride,
+                                                sqr_threshold, mask);
+      });
+    }
+    return rcs[(size_t)r];
+  });
+  if (rc == GICPB_E_BADARG)  // a bad cloud (no finite point) fails on every rank: report it as one context does
+    for (size_t r = 0; r < rcs.size(); ++r)
+      if (rcs[r] == GICPB_E_BADARG) {
+        g->err = g->ctx[r]->err;
+        break;
+      }
+  if (rc == GICPB_OK && n_kept) {
+    unsigned long long total = 0;
+    for (unsigned long long k : kept) total += k;
+    *n_kept = (int64_t)total;
+  }
   return rc;
 }
 

@@ -109,8 +109,11 @@ class GridIndex {
   // in it (knn_window() tells the kNN kernel where the window ends; it reports every point it cannot vouch for, and the
   // caller then widens the window to the whole cloud with widen()).  Same grid geometry, keys and order as the whole
   // cloud's index: the window IS that index cut to its planes (bricks are numbered plane by plane for this).
+  // halo_m >= 0 (the SUBTRACT cloud of a group's difference): the halo is as many planes as cover a search radius of halo_m
+  // metres from any point of the rank's own planes (GICPB_HALO_PLANES does not apply); INFINITY: the whole cloud.
   void build(const void* raw, int64_t n, int64_t stride_bytes, bool on_device, float cell_size,
-             float points_per_cell, cudaStream_t stream, HostStager* stager = nullptr, int rank = 0, int world = 1);
+             float points_per_cell, cudaStream_t stream, HostStager* stager = nullptr, int rank = 0, int world = 1,
+             double halo_m = -1.0);
   void widen(cudaStream_t stream);  // re-index with the window = the whole cloud (the shard stays the same set of points)
   bool windowed() const { return win_.active && !(win_.w_lo == 0 && win_.w_hi == win_.planes); }
   bool plane_sharded() const { return win_.active; }  // the shard is a range of brick planes (else: an index range)
@@ -122,6 +125,12 @@ class GridIndex {
     float lo = 0.f, hi = 0.f;
   };
   KnnWindow knn_window() const;
+  // plane_sharded(): the finite rows of a query cloud (raw, n, stride: xyz floats) whose brick plane on this grid - clamped to
+  // the grid as the build clamps - is one of the rank's own planes, in row order, as float4 rows (x, y, z, w = row index as int
+  // bits); returns how many.  Ownership partitions the finite rows over the ranks.  flags / pos hold n + 1 words, tmp
+  // scan_tmp_entries(n + 1).  Synchronises `stream`.
+  int64_t owned_queries(const unsigned char* raw, int64_t n, int64_t stride, float4* out, uint32_t* flags, uint32_t* pos,
+                        uint32_t* tmp, cudaStream_t stream) const;
   bool ready() const { return ready_; }
   const GridView& view() const { return view_; }
   const Info& info() const { return info_; }
@@ -180,6 +189,11 @@ class GridIndex {
 // (gicpb_set_clouds); called once per context
 void prefer_shared_carveout_grid();
 void prefer_shared_carveout_sort();
+
+// cloud difference over a group (grid_build.cu): keep[j] of the routed rows -> full[row index in rows[j].w]
+void scatter_keep(const float4* rows, const unsigned char* keep, int64_t n_rows, unsigned char* full, cudaStream_t stream);
+// out[i] = OR over r < n_parts of parts[r * len + i]
+void or_parts(const unsigned char* parts, int n_parts, int64_t len, unsigned char* out, cudaStream_t stream);
 
 // hand-written device-wide primitives (sort_scan.cu)
 size_t scan_tmp_entries(int64_t n);

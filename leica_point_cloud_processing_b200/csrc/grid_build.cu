@@ -230,6 +230,46 @@ __global__ void __launch_bounds__(256) window_gather_kernel(const float4* __rest
   if (i < n && flags[i]) out[pos[i]] = pts[i];
 }
 
+// ---- cloud difference over a group: the input rows whose brick plane (on the subtract's grid) a rank owns -----------------
+__global__ void __launch_bounds__(256) route_flags_kernel(const unsigned char* __restrict__ raw, int64_t n, int64_t stride,
+                                                           GridView g, int axis, int own_lo, int own_hi,
+                                                           uint32_t* __restrict__ flags) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float* p = reinterpret_cast<const float*>(raw + i * stride);
+  const float4 q = make_float4(p[0], p[1], p[2], 0.f);
+  bool in = false;
+  if (finite3(q.x, q.y, q.z)) {
+    const int pl = plane_of(g, axis, q);
+    in = pl >= own_lo && pl < own_hi;
+  }
+  flags[i] = in ? 1u : 0u;
+}
+
+__global__ void __launch_bounds__(256) route_gather_kernel(const unsigned char* __restrict__ raw, int64_t n, int64_t stride,
+                                                            const uint32_t* __restrict__ flags,
+                                                            const uint32_t* __restrict__ pos, float4* __restrict__ out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n || !flags[i]) return;
+  const float* p = reinterpret_cast<const float*>(raw + i * stride);
+  out[pos[i]] = make_float4(p[0], p[1], p[2], __int_as_float((int)i));
+}
+
+__global__ void __launch_bounds__(256) scatter_keep_kernel(const float4* __restrict__ rows, const unsigned char* __restrict__ keep,
+                                                            int64_t n_rows, unsigned char* __restrict__ full) {
+  const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < n_rows) full[__float_as_int(rows[j].w)] = keep[j];
+}
+
+__global__ void __launch_bounds__(256) or_parts_kernel(const unsigned char* __restrict__ parts, int n_parts, int64_t len,
+                                                        unsigned char* __restrict__ out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= len) return;
+  unsigned char v = 0;
+  for (int r = 0; r < n_parts; ++r) v |= parts[(int64_t)r * len + i];
+  out[i] = v;
+}
+
 // brick table from the occupancy marks (rank = exclusive scan of occ): slot = rank of the brick among the occupied bricks
 // (so slots ascend with the brick index), -1 for an empty brick; the brick's bit in its superbrick mask and the
 // superbrick's bit in its hyperbrick mask; scratch[7] = number of occupied bricks
@@ -594,8 +634,20 @@ static int halo_planes() {
   return v;
 }
 
+// Halo of the subtract cloud's window (halo_m = the search radius sqrt(thr_next) of a difference).  A subtract point s that can
+// hit a query q (float d2 < thr_next) has |s_a - q_a| <= halo_m along the split axis, up to the rounding of the float
+// distance, which the grid's margin covers (it is the slack of every box bound of the searches).  cell_of is monotone in the
+// coordinate, and floor() plus the rounding of (v - o) * inv_h move a cell index by less than one cell, so
+// cell(s) < cell(q) + (halo_m + margin) / h + 1.  A query the rank owns has cell(q) < 8 own_hi, hence cell(s) < 8 (own_hi + H)
+// - plane(s) < own_hi + H, inside the window - as soon as 8 h H >= halo_m + margin + h; the same holds below own_lo.  A query
+// outside the grid is clamped to an end plane, and the points near it lie in the first (last) planes, in that window too.
+static int difference_halo(double halo_m, double h, double margin, int planes) {
+  const double H = std::ceil((halo_m + margin + h) / (8.0 * h));
+  return H < (double)planes ? std::max(1, (int)H) : planes;  // INFINITY: the whole cloud
+}
+
 void GridIndex::build(const void* raw, int64_t n, int64_t stride_bytes, bool on_device, float cell_size,
-                      float points_per_cell, cudaStream_t stream, HostStager* stager, int rank, int world) {
+                      float points_per_cell, cudaStream_t stream, HostStager* stager, int rank, int world, double halo_m) {
   const auto t_begin = std::chrono::steady_clock::now();
   BuildTrace trace(stream);
   trace.mark("begin");
@@ -798,7 +850,8 @@ void GridIndex::build(const void* raw, int64_t n, int64_t stride_bytes, bool on_
         win_.planes = planes;
         win_.own_lo = cut(rank);
         win_.own_hi = cut(rank + 1);
-        set_window(std::max(0, win_.own_lo - halo_planes()), std::min(planes, win_.own_hi + halo_planes()));
+        const int halo = halo_m >= 0 ? difference_halo(halo_m, g.h, g.margin, planes) : halo_planes();
+        set_window(std::max(0, win_.own_lo - halo), std::min(planes, win_.own_hi + halo));
       } else {  // degenerate split: index everything, shards by index range (the default numbering again)
         g.bsx = 1; g.bsy = bd[0]; g.bsz = bd[0] * bd[1];
         g.bo0 = 0; g.bo1 = 1; g.bo2 = 2;
@@ -854,6 +907,33 @@ const float4* GridIndex::window_points(cudaStream_t stream, int64_t* n_local) {
                                                               pts_local_.get());
   GICPB_LAUNCHED();
   return pts_local_.get();
+}
+
+int64_t GridIndex::owned_queries(const unsigned char* raw, int64_t n, int64_t stride, float4* out, uint32_t* flags,
+                                 uint32_t* pos, uint32_t* tmp, cudaStream_t stream) const {
+  // flags[n] = 0: the exclusive scan leaves the number of owned rows in pos[n]
+  GICPB_CUDA(cudaMemsetAsync(flags + n, 0, sizeof(uint32_t), stream));
+  route_flags_kernel<<<blocks_for(n, 256), 256, 0, stream>>>(raw, n, stride, geom_, win_.axis, win_.own_lo, win_.own_hi, flags);
+  GICPB_LAUNCHED();
+  exclusive_scan_u32(flags, pos, n + 1, tmp, stream);
+  route_gather_kernel<<<blocks_for(n, 256), 256, 0, stream>>>(raw, n, stride, flags, pos, out);
+  GICPB_LAUNCHED();
+  uint32_t owned = 0;
+  GICPB_CUDA(cudaMemcpyAsync(&owned, pos + n, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+  GICPB_CUDA(cudaStreamSynchronize(stream));
+  return (int64_t)owned;
+}
+
+void scatter_keep(const float4* rows, const unsigned char* keep, int64_t n_rows, unsigned char* full, cudaStream_t stream) {
+  if (n_rows <= 0) return;
+  scatter_keep_kernel<<<blocks_for(n_rows, 256), 256, 0, stream>>>(rows, keep, n_rows, full);
+  GICPB_LAUNCHED();
+}
+
+void or_parts(const unsigned char* parts, int n_parts, int64_t len, unsigned char* out, cudaStream_t stream) {
+  if (len <= 0) return;
+  or_parts_kernel<<<blocks_for(len, 256), 256, 0, stream>>>(parts, n_parts, len, out);
+  GICPB_LAUNCHED();
 }
 
 void GridIndex::widen(cudaStream_t stream) {

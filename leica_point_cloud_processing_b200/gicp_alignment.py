@@ -206,6 +206,7 @@ class GICPAlignment:
 def remove_from_cloud(input_cloud, subtract_cloud, threshold, engine=None, device=0):
     """Filter::removeFromCloud (reference src/Filter.cpp:176-189): the points of `input_cloud` whose SQUARED
     distance to their nearest neighbour in `subtract_cloud` exceeds `threshold`, in input order.
+    `engine` may be an EngineGroup (host clouds): the difference then runs on all of its GPUs.
     Returns (filtered_cloud, mask)."""
     eng = engine if engine is not None else Engine(device)
     log.info("Difference from segment with threshold: %f", threshold)
