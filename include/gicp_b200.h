@@ -233,8 +233,10 @@ int gicpb_euclidean_clusters(gicpb_ctx* ctx, const void* cloud, int64_t n, int64
  * downsampled): one point per occupied voxel, in ascending voxel index (PCL's output order): xyz = mean of the
  * voxel's points (float sums), stride >= 16: data[3] = 1, stride >= 20: the rgba word at byte 16 = per-channel
  * mean (truncated), all other bytes 0 (the last input point must extend through its rgba word).  `out` must have room for n points of the same stride (host or device like
- * `in`).  When the voxel indices would overflow 32 bits PCL warns and passes the input through: so does this call
- * (n_out = n, the warning is left in gicpb_last_error). */
+ * `in`); every byte of the n_out rows is written.  When PCL's check refuses the leaf (dx * dy * dz > INT32_MAX with
+ * d = int((max - min) / leaf) + 1) PCL warns and passes the input through: so does this call (n_out = n, the warning
+ * is left in gicpb_last_error; a call that downsamples leaves gicpb_last_error empty).  Past that check PCL's 32-bit
+ * voxel index may wrap; the output then matches PCL's, which averages the voxels that share a wrapped index. */
 int gicpb_voxel_grid(gicpb_ctx* ctx, const void* in, int64_t n, int64_t stride_bytes, int on_device, double leaf_size,
                      void* out, int64_t* n_out);
 

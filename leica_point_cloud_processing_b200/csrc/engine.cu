@@ -1955,6 +1955,7 @@ int gicpb_voxel_grid(gicpb_ctx* c, const void* in, int64_t n, int64_t stride, in
   return guarded(c, [&] {
     if (!n_out) throw ArgError("null n_out");
     *n_out = 0;
+    c->err.clear();  // the overflow warning below is the only text a successful call leaves
     if (n == 0) return;
     if (!out) throw ArgError("null output");
     check_cloud_args(in, n, stride);
@@ -1985,8 +1986,7 @@ int gicpb_voxel_grid(gicpb_ctx* c, const void* in, int64_t n, int64_t stride, in
       *n_out = n;
       return;
     }
-    if (!on_device && m > 0)
-      download_bytes(c, out, d_out, (size_t)(m - 1) * stride + std::min<size_t>((size_t)stride, 20));
+    if (!on_device && m > 0) download_bytes(c, out, d_out, (size_t)m * stride);  // whole rows: the zero bytes too
     GICPB_CUDA(cudaStreamSynchronize(c->stream));
     *n_out = m;
   });

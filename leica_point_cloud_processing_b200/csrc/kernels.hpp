@@ -203,7 +203,8 @@ void launch_cluster_unions(const GridView& g, float r2, int* parent, int* root_o
 
 // pcl::VoxelGrid::applyFilter on strided points (xyz first; rgba word at byte 16 when stride >= 20).  Writes one
 // centroid point per occupied voxel to d_out (ascending voxel index, same stride) and returns their number.
-// *overflow: the voxel indices would not fit 32 bits ("leaf size too small"): nothing is written, n is returned.
+// *overflow: PCL's check dx * dy * dz > INT32_MAX refuses the leaf ("leaf size too small"): nothing is written, n is
+// returned.
 class VoxelGrid {
  public:
   int64_t run(const unsigned char* d_in, int64_t n, int64_t stride, float leaf, unsigned char* d_out, cudaStream_t stream,

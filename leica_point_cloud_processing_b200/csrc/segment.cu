@@ -184,26 +184,34 @@ __global__ void __launch_bounds__(256) voxel_minmax_kernel(const unsigned char* 
 struct VoxelParams {
   float inv_leaf[3];
   int min_b[3];
-  int mul[3];  // divb_mul_: 1, div0, div0 * div1
+  uint32_t mul[3];  // divb_mul_: 1, div0, div0 * div1 (wrapped to 32 bits, as PCL's int product)
 };
 
-// voxel_grid.hpp first pass: ijk = int(floor(x * inverse_leaf) - float(min_b)); idx = ijk . divb_mul
+__global__ void __launch_bounds__(256) voxel_finite_kernel(const unsigned char* __restrict__ raw, int64_t n, int64_t stride,
+                                                            uint32_t* __restrict__ flags) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float* p = reinterpret_cast<const float*>(raw + i * stride);
+  flags[i] = finite3(p[0], p[1], p[2]) ? 1u : 0u;
+}
+
+// voxel_grid.hpp first pass: ijk = int(floor(x * inverse_leaf) - float(min_b)); idx = ijk . divb_mul in 32-bit
+// arithmetic that wraps as PCL's int index does.  The finite points land at pos[i] (the exclusive scan of
+// voxel_finite_kernel's flags), or at i when every point is finite (pos == nullptr).
 __global__ void __launch_bounds__(256) voxel_keys_kernel(const unsigned char* __restrict__ raw, int64_t n, int64_t stride,
-                                                          VoxelParams vp, uint32_t sentinel, uint32_t* __restrict__ keys,
-                                                          uint32_t* __restrict__ vals) {
+                                                          VoxelParams vp, const uint32_t* __restrict__ pos,
+                                                          uint32_t* __restrict__ keys, uint32_t* __restrict__ vals) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float* p = reinterpret_cast<const float*>(raw + i * stride);
   const float x = p[0], y = p[1], z = p[2];
-  uint32_t key = sentinel;
-  if (finite3(x, y, z)) {
-    const int i0 = __float2int_rz(__fsub_rn(floorf(__fmul_rn(x, vp.inv_leaf[0])), (float)vp.min_b[0]));
-    const int i1 = __float2int_rz(__fsub_rn(floorf(__fmul_rn(y, vp.inv_leaf[1])), (float)vp.min_b[1]));
-    const int i2 = __float2int_rz(__fsub_rn(floorf(__fmul_rn(z, vp.inv_leaf[2])), (float)vp.min_b[2]));
-    key = (uint32_t)(i0 * vp.mul[0] + i1 * vp.mul[1] + i2 * vp.mul[2]);
-  }
-  keys[i] = key;
-  vals[i] = (uint32_t)i;
+  if (!finite3(x, y, z)) return;
+  const int i0 = __float2int_rz(__fsub_rn(floorf(__fmul_rn(x, vp.inv_leaf[0])), (float)vp.min_b[0]));
+  const int i1 = __float2int_rz(__fsub_rn(floorf(__fmul_rn(y, vp.inv_leaf[1])), (float)vp.min_b[1]));
+  const int i2 = __float2int_rz(__fsub_rn(floorf(__fmul_rn(z, vp.inv_leaf[2])), (float)vp.min_b[2]));
+  const uint32_t j = pos ? pos[i] : (uint32_t)i;
+  keys[j] = (uint32_t)i0 * vp.mul[0] + (uint32_t)i1 * vp.mul[1] + (uint32_t)i2 * vp.mul[2];
+  vals[j] = (uint32_t)i;
 }
 
 __global__ void __launch_bounds__(256) voxel_heads_kernel(const uint32_t* __restrict__ keys, int n_valid,
@@ -308,7 +316,7 @@ int64_t VoxelGrid::run(const unsigned char* d_in, int64_t n, int64_t stride, flo
   float min_p[3], max_p[3];
   int64_t cells = 1;
   VoxelParams vp{};
-  int div[3];
+  int64_t div[3];
   for (int a = 0; a < 3; ++a) {
     min_p[a] = ord2f(hs[a]);
     max_p[a] = ord2f(hs[3 + a]);
@@ -319,29 +327,37 @@ int64_t VoxelGrid::run(const unsigned char* d_in, int64_t n, int64_t stride, flo
       return n;
     }
   }
+  // div_b can exceed dx by one on every axis, so div0 * div1 * div2 may pass 2^31 and even 2^32 where PCL's check
+  // passes; PCL's 32-bit index then wraps and voxels that share the wrapped index are averaged together.
+  bool wide = false;  // an index may reach 2^24 voxels along an axis, where float(ijk) rounds: sort on all 32 bits
+  double total = 1.0;
   for (int a = 0; a < 3; ++a) {
     vp.inv_leaf[a] = inv;
     vp.min_b[a] = (int)std::floor(min_p[a] * inv);
-    const int max_b = (int)std::floor(max_p[a] * inv);
+    const int64_t max_b = (int64_t)std::floor(max_p[a] * inv);
     div[a] = max_b - vp.min_b[a] + 1;
+    wide = wide || div[a] > (1 << 24);
+    total *= (double)div[a];
   }
-  vp.mul[0] = 1;
-  vp.mul[1] = div[0];
-  vp.mul[2] = div[0] * div[1];
-  const int64_t total = (int64_t)div[0] * div[1] * div[2];
-  if (total > (int64_t)INT32_MAX) {  // cannot happen after the check above, kept for safety of the 32-bit keys
-    *overflow = true;
-    return n;
-  }
-  const uint32_t sentinel = (uint32_t)total;
-  int key_bits = 1;
-  while ((1ull << key_bits) <= (unsigned long long)sentinel) ++key_bits;
+  vp.mul[0] = 1u;
+  vp.mul[1] = (uint32_t)div[0];
+  vp.mul[2] = (uint32_t)div[0] * (uint32_t)div[1];
+  int key_bits = 1;  // the keys are below total
+  while (key_bits < 32 && (wide || (double)(1ull << key_bits) < total)) ++key_bits;
   keys_a_.reserve(n); keys_b_.reserve(n); vals_a_.reserve(n); vals_b_.reserve(n);
   scan_tmp_.reserve(scan_tmp_entries(n));
-  sorter_.prepare(n, stream);
-  voxel_keys_kernel<<<nblk(n, 256), 256, 0, stream>>>(d_in, n, stride, vp, sentinel, keys_a_.get(), vals_a_.get());
+  sorter_.prepare(n_valid, stream);
+  const uint32_t* pos = nullptr;
+  if (n_valid < n) {  // compact the finite points, in input order, so that every 32-bit key is a voxel index
+    voxel_finite_kernel<<<nblk(n, 256), 256, 0, stream>>>(d_in, n, stride, keys_b_.get());
+    GICPB_LAUNCHED();
+    exclusive_scan_u32(keys_b_.get(), vals_b_.get(), n, scan_tmp_.get(), stream);
+    pos = vals_b_.get();
+  }
+  voxel_keys_kernel<<<nblk(n, 256), 256, 0, stream>>>(d_in, n, stride, vp, pos, keys_a_.get(), vals_a_.get());
   GICPB_LAUNCHED();
-  const bool in_b = sorter_.sort(keys_a_.get(), vals_a_.get(), keys_b_.get(), vals_b_.get(), n, key_bits, false, stream);
+  const bool in_b = sorter_.sort(keys_a_.get(), vals_a_.get(), keys_b_.get(), vals_b_.get(), n_valid, key_bits, false,
+                                 stream);
   const uint32_t* skeys = in_b ? keys_b_.get() : keys_a_.get();
   const uint32_t* svals = in_b ? vals_b_.get() : vals_a_.get();
   uint32_t* flags = in_b ? keys_a_.get() : keys_b_.get();

@@ -1634,7 +1634,9 @@ int64_t orc_voxel_grid(const unsigned char* pts, int64_t n, int64_t stride, doub
     const int max_b = (int)std::floor(max_p[a] * inv);
     div_b[a] = max_b - min_b[a] + 1;
   }
-  const int mul[3] = {1, div_b[0], div_b[0] * div_b[1]};
+  // PCL's int index arithmetic, in uint32_t so that it wraps with the same bits where div_b[0] * div_b[1] * div_b[2]
+  // passes 2^31 (its dx * dy * dz check can pass while div_b, up to dx + 1 per axis, does not)
+  const uint32_t mul[3] = {1u, (uint32_t)div_b[0], (uint32_t)div_b[0] * (uint32_t)div_b[1]};
   std::vector<std::pair<unsigned, int64_t>> index_vector;
   index_vector.reserve((size_t)n_valid);
   for (int64_t i = 0; i < n; ++i) {
@@ -1643,7 +1645,7 @@ int64_t orc_voxel_grid(const unsigned char* pts, int64_t n, int64_t stride, doub
     const int ijk0 = (int)(std::floor(p[0] * inv) - (float)min_b[0]);
     const int ijk1 = (int)(std::floor(p[1] * inv) - (float)min_b[1]);
     const int ijk2 = (int)(std::floor(p[2] * inv) - (float)min_b[2]);
-    index_vector.emplace_back((unsigned)(ijk0 * mul[0] + ijk1 * mul[1] + ijk2 * mul[2]), i);
+    index_vector.emplace_back((uint32_t)ijk0 * mul[0] + (uint32_t)ijk1 * mul[1] + (uint32_t)ijk2 * mul[2], i);
   }
   std::stable_sort(index_vector.begin(), index_vector.end(),
                    [](const std::pair<unsigned, int64_t>& a, const std::pair<unsigned, int64_t>& b) { return a.first < b.first; });

@@ -171,7 +171,9 @@ def test_reference_testFODClustering(engine, oracle):
     (1, 20000, 0.02, 1, 0),        # sparse: mostly singletons
     (2, 20000, 0.05, 3, 0),        # mixed
     (3, 20000, 0.05, 3, 40),       # upper size limit
-    (4, 3000, 0.6, 1, 0),          # tolerance >> spacing: balls span many cells (hierarchical search), one cluster
+    (4, 3000, 0.6, 1, 0),          # tolerance >> spacing: one cluster (the cell is never smaller than the tolerance,
+                                   # so each ball spans a few cells: near search only; the far search runs where
+                                   # the box margin grows with |x|, see test_segment_edges.py)
 ])
 def test_clusters_match_oracle_random(engine, oracle, seed, n, tol, min_size, max_size):
     rng = np.random.default_rng(seed)
