@@ -1421,11 +1421,13 @@ void roots2_f(float b, float c, float roots[3]) {
   roots[2] = 0.5f * (b + sd);
   roots[1] = 0.5f * (b - sd);
 }
-void roots3_f(const float m[9], float roots[3]) {
+// *branch: 2 = c0 < epsilon -> roots2, 3 = trigonometric roots, 4 = trigonometric roots, then the roots2 fallback
+void roots3_f(const float m[9], float roots[3], int* branch) {
   const float c0 = m[0] * m[4] * m[8] + 2.f * m[1] * m[2] * m[5] - m[0] * m[5] * m[5] - m[4] * m[2] * m[2] - m[8] * m[1] * m[1];
   const float c1 = m[0] * m[4] - m[1] * m[1] + m[0] * m[8] - m[2] * m[2] + m[4] * m[8] - m[5] * m[5];
   const float c2 = m[0] + m[4] + m[8];
   if (std::fabs(c0) < std::numeric_limits<float>::epsilon()) {
+    *branch = 2;
     roots2_f(c2, c1, roots);
     return;
   }
@@ -1448,108 +1450,131 @@ void roots3_f(const float m[9], float roots[3]) {
     std::swap(roots[1], roots[2]);
     if (roots[0] >= roots[1]) std::swap(roots[0], roots[1]);
   }
-  if (roots[0] <= 0.f) roots2_f(c2, c1, roots);
+  *branch = 3;
+  if (roots[0] <= 0.f) {
+    *branch = 4;
+    roots2_f(c2, c1, roots);
+  }
 }
-}  // namespace
 
-int orc_normals(const float* xyz, int n, double radius, float* out4) {
+// the normal of point i into o[0..3]; info (may be null): neighbour count, branch (0 no normal: non-finite point or < 3
+// neighbours; 1 zero covariance: every |entry| <= FLT_MIN; 2..4 as roots3_f), root gap roots[1] - roots[0] of the scaled
+// matrix, cos_theta of the viewpoint flip.  Returns whether the normal is finite.
+bool normal_at(const KdTree& tree, const float* xyz, int i, float r2, float* o, double* info) {
+  const float nan = std::numeric_limits<float>::quiet_NaN();
+  o[0] = o[1] = o[2] = o[3] = nan;
+  if (info) info[0] = info[1] = 0.0, info[2] = info[3] = nan;
+  const float* p = xyz + 3 * i;
+  if (!(std::isfinite(p[0]) && std::isfinite(p[1]) && std::isfinite(p[2]))) return false;
+  std::vector<int> nn;
+  tree.radius(p, r2, nn);
+  if (info) info[0] = (double)nn.size();
+  if (nn.size() < 3) return false;
+  std::vector<std::pair<float, int>> order;
+  order.reserve(nn.size());
+  for (int j : nn) order.emplace_back(sqdist(p, xyz + 3 * j), j);
+  std::sort(order.begin(), order.end());
+  float accu[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  for (const auto& e : order) {
+    const float* c = xyz + 3 * e.second;
+    accu[0] += c[0] * c[0];
+    accu[1] += c[0] * c[1];
+    accu[2] += c[0] * c[2];
+    accu[3] += c[1] * c[1];
+    accu[4] += c[1] * c[2];
+    accu[5] += c[2] * c[2];
+    accu[6] += c[0];
+    accu[7] += c[1];
+    accu[8] += c[2];
+  }
+  const float cntf = (float)order.size();
+  for (int k = 0; k < 9; ++k) accu[k] /= cntf;
+  float m[9];
+  m[0] = accu[0] - accu[6] * accu[6];
+  m[1] = accu[1] - accu[6] * accu[7];
+  m[2] = accu[2] - accu[6] * accu[8];
+  m[4] = accu[3] - accu[7] * accu[7];
+  m[5] = accu[4] - accu[7] * accu[8];
+  m[8] = accu[5] - accu[8] * accu[8];
+  m[3] = m[1];
+  m[6] = m[2];
+  m[7] = m[5];
+  // pcl::eigen33(mat, eigenvalue, eigenvector)
+  float scale = 0.f;
+  for (int k = 0; k < 9; ++k) scale = std::max(scale, std::fabs(m[k]));
+  const bool zero_cov = scale <= std::numeric_limits<float>::min();
+  if (zero_cov) scale = 1.f;
+  float sm[9];
+  for (int k = 0; k < 9; ++k) sm[k] = m[k] / scale;
+  float roots[3];
+  int branch = 0;
+  roots3_f(sm, roots, &branch);
+  if (info) info[1] = zero_cov ? 1 : branch, info[2] = (double)roots[1] - (double)roots[0];
+  const float eigenvalue = roots[0] * scale;
+  sm[0] -= roots[0];
+  sm[4] -= roots[0];
+  sm[8] -= roots[0];
+  auto cross = [](const float* a, const float* b, float* c) {
+    c[0] = a[1] * b[2] - a[2] * b[1];
+    c[1] = a[2] * b[0] - a[0] * b[2];
+    c[2] = a[0] * b[1] - a[1] * b[0];
+  };
+  float v1[3], v2[3], v3[3];
+  cross(sm, sm + 3, v1);
+  cross(sm, sm + 6, v2);
+  cross(sm + 3, sm + 6, v3);
+  const float l1 = v1[0] * v1[0] + v1[1] * v1[1] + v1[2] * v1[2];
+  const float l2 = v2[0] * v2[0] + v2[1] * v2[1] + v2[2] * v2[2];
+  const float l3 = v3[0] * v3[0] + v3[1] * v3[1] + v3[2] * v3[2];
+  const float* v = v3;
+  float len = l3;
+  if (l1 >= l2 && l1 >= l3) {
+    v = v1;
+    len = l1;
+  } else if (l2 >= l1 && l2 >= l3) {
+    v = v2;
+    len = l2;
+  }
+  const float s = std::sqrt(len);
+  float nx = v[0] / s, ny = v[1] / s, nz = v[2] / s;
+  const float eig_sum = m[0] + m[4] + m[8];
+  const float curvature = eig_sum != 0.f ? std::fabs(eigenvalue / eig_sum) : 0.f;
+  // flipNormalTowardsViewpoint(point, 0, 0, 0, ...)
+  const float vx = 0.f - p[0], vy = 0.f - p[1], vz = 0.f - p[2];
+  const float cos_theta = vx * nx + vy * ny + vz * nz;
+  if (info) info[3] = cos_theta;
+  if (cos_theta < 0) {
+    nx *= -1;
+    ny *= -1;
+    nz *= -1;
+  }
+  o[0] = nx;
+  o[1] = ny;
+  o[2] = nz;
+  o[3] = curvature;
+  // a covariance that cancelled to zero gives 0 / 0 above: the normal is NaN although the point has neighbours
+  return std::isfinite(nx) && std::isfinite(ny) && std::isfinite(nz);
+}
+
+int normals_impl(const float* xyz, int n, double radius, float* out4, double* info4) {
   KdTree tree(xyz, n);
   const float r2 = (float)(radius * radius);
-  const float nan = std::numeric_limits<float>::quiet_NaN();
   int kept = 0;
 #ifdef _OPENMP
 #pragma omp parallel for reduction(+ : kept) schedule(dynamic, 256)
 #endif
-  for (int i = 0; i < n; ++i) {
-    float* o = out4 + 4 * (size_t)i;
-    o[0] = o[1] = o[2] = o[3] = nan;
-    const float* p = xyz + 3 * i;
-    if (!(std::isfinite(p[0]) && std::isfinite(p[1]) && std::isfinite(p[2]))) continue;
-    std::vector<int> nn;
-    tree.radius(p, r2, nn);
-    if (nn.size() < 3) continue;
-    std::vector<std::pair<float, int>> order;
-    order.reserve(nn.size());
-    for (int j : nn) order.emplace_back(sqdist(p, xyz + 3 * j), j);
-    std::sort(order.begin(), order.end());
-    float accu[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-    for (const auto& e : order) {
-      const float* c = xyz + 3 * e.second;
-      accu[0] += c[0] * c[0];
-      accu[1] += c[0] * c[1];
-      accu[2] += c[0] * c[2];
-      accu[3] += c[1] * c[1];
-      accu[4] += c[1] * c[2];
-      accu[5] += c[2] * c[2];
-      accu[6] += c[0];
-      accu[7] += c[1];
-      accu[8] += c[2];
-    }
-    const float cntf = (float)order.size();
-    for (int k = 0; k < 9; ++k) accu[k] /= cntf;
-    float m[9];
-    m[0] = accu[0] - accu[6] * accu[6];
-    m[1] = accu[1] - accu[6] * accu[7];
-    m[2] = accu[2] - accu[6] * accu[8];
-    m[4] = accu[3] - accu[7] * accu[7];
-    m[5] = accu[4] - accu[7] * accu[8];
-    m[8] = accu[5] - accu[8] * accu[8];
-    m[3] = m[1];
-    m[6] = m[2];
-    m[7] = m[5];
-    // pcl::eigen33(mat, eigenvalue, eigenvector)
-    float scale = 0.f;
-    for (int k = 0; k < 9; ++k) scale = std::max(scale, std::fabs(m[k]));
-    if (scale <= std::numeric_limits<float>::min()) scale = 1.f;
-    float sm[9];
-    for (int k = 0; k < 9; ++k) sm[k] = m[k] / scale;
-    float roots[3];
-    roots3_f(sm, roots);
-    const float eigenvalue = roots[0] * scale;
-    sm[0] -= roots[0];
-    sm[4] -= roots[0];
-    sm[8] -= roots[0];
-    auto cross = [](const float* a, const float* b, float* c) {
-      c[0] = a[1] * b[2] - a[2] * b[1];
-      c[1] = a[2] * b[0] - a[0] * b[2];
-      c[2] = a[0] * b[1] - a[1] * b[0];
-    };
-    float v1[3], v2[3], v3[3];
-    cross(sm, sm + 3, v1);
-    cross(sm, sm + 6, v2);
-    cross(sm + 3, sm + 6, v3);
-    const float l1 = v1[0] * v1[0] + v1[1] * v1[1] + v1[2] * v1[2];
-    const float l2 = v2[0] * v2[0] + v2[1] * v2[1] + v2[2] * v2[2];
-    const float l3 = v3[0] * v3[0] + v3[1] * v3[1] + v3[2] * v3[2];
-    const float* v = v3;
-    float len = l3;
-    if (l1 >= l2 && l1 >= l3) {
-      v = v1;
-      len = l1;
-    } else if (l2 >= l1 && l2 >= l3) {
-      v = v2;
-      len = l2;
-    }
-    const float s = std::sqrt(len);
-    float nx = v[0] / s, ny = v[1] / s, nz = v[2] / s;
-    const float eig_sum = m[0] + m[4] + m[8];
-    const float curvature = eig_sum != 0.f ? std::fabs(eigenvalue / eig_sum) : 0.f;
-    // flipNormalTowardsViewpoint(point, 0, 0, 0, ...)
-    const float vx = 0.f - p[0], vy = 0.f - p[1], vz = 0.f - p[2];
-    const float cos_theta = vx * nx + vy * ny + vz * nz;
-    if (cos_theta < 0) {
-      nx *= -1;
-      ny *= -1;
-      nz *= -1;
-    }
-    o[0] = nx;
-    o[1] = ny;
-    o[2] = nz;
-    o[3] = curvature;
-    // a covariance that cancelled to zero gives 0 / 0 above: the normal is NaN although the point has neighbours
-    kept += (std::isfinite(nx) && std::isfinite(ny) && std::isfinite(nz)) ? 1 : 0;
-  }
+  for (int i = 0; i < n; ++i)
+    kept += normal_at(tree, xyz, i, r2, out4 + 4 * (size_t)i, info4 ? info4 + 4 * (size_t)i : nullptr) ? 1 : 0;
   return kept;
+}
+}  // namespace
+
+int orc_normals(const float* xyz, int n, double radius, float* out4) { return normals_impl(xyz, n, radius, out4, nullptr); }
+
+// orc_normals plus, per point, info4 = (neighbour count, branch, root gap, cos_theta) - see normal_at.  The rows of out4 are
+// the rows orc_normals gives.
+int orc_normals_ex(const float* xyz, int n, double radius, float* out4, double* info4) {
+  return normals_impl(xyz, n, radius, out4, info4);
 }
 
 // ---- pcl::EuclideanClusterExtraction::extract (reference src/FODDetector.cpp:45-58): extractEuclideanClusters

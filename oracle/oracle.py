@@ -229,6 +229,19 @@ class Oracle:
         n = self.lib.orc_normals(_p(a, c_float_p), ctypes.c_int(len(a)), ctypes.c_double(radius), _p(out, c_float_p))
         return out, int(n)
 
+    def normals_ex(self, xyz, radius):
+        """normals() plus float64 [n, 4] info per point: neighbour count; branch (0 no normal: non-finite point or < 3
+        neighbours, 1 zero covariance, 2 pcl::eigen33's c0 < eps -> roots2, 3 trigonometric roots, 4 trigonometric roots
+        then the roots2 fallback); root gap roots[1] - roots[0] of the scaled matrix; cos_theta of the viewpoint flip.
+        Returns (rows, info, finite count); the rows are the rows normals() gives."""
+        a = _xyz(xyz)
+        out = np.empty((len(a), 4), np.float32)
+        info = np.empty((len(a), 4), np.float64)
+        self.lib.orc_normals_ex.restype = ctypes.c_int
+        n = self.lib.orc_normals_ex(_p(a, c_float_p), ctypes.c_int(len(a)), ctypes.c_double(radius), _p(out, c_float_p),
+                                    _p(info, c_double_p))
+        return out, info, int(n)
+
     def euclidean_clusters(self, xyz, tolerance, min_size=1, max_size=0):
         """pcl::EuclideanClusterExtraction::extract: (labels in PCL's cluster order, -1 = none; n_clusters)"""
         a = _xyz(xyz) if len(xyz) else np.zeros((0, 3), np.float32)
