@@ -42,6 +42,12 @@ constexpr int kMaxBoxRows = 81;                 // NN-1: largest (y,z) row count
 constexpr int kSeedBoxRows = 4;                 // NN-1: a seed whose ball spans more rows is first improved by a probe
 constexpr int kNearMaxRing = 3;                // NN-1: cell rings probed for a first candidate before the far search
 constexpr int kKnnMaxRing = 4;                  // kNN: largest cell ring searched before the hierarchical fallback
+// Point ranges a thread can queue before it scans them (QueueVisitor), as the kernels instantiate the near searches;
+// tests/host_emul builds the same instances.  NN-1 (nn_kernels.cu): 3x3 rows, one of them split by a brick edge; 16
+// entries took 16 KB of every block from L1: correspondence kernels of a job 1.616 -> 1.58 ms at 1 M, 27.5 -> 26.5 ms
+// at 8 M.  kNN (knn_cov.cu): in dynamic shared memory beside the k-best lists.
+constexpr int kNnQueueCap = 10;
+constexpr int kKnnQueueCap = 8;
 constexpr unsigned kFullMask = 0xffffffffu;
 
 // ---- arithmetic with one rounding per operation on both sides (bit-exact against the oracle) -------------------------

@@ -55,8 +55,6 @@ __device__ __forceinline__ void jacobi_rotate(double (&a)[9], double (&v)[9]) {
   }
 }
 
-constexpr int kKnnQueueCap = 8;
-
 template <bool kFar, int kKnnThreads>
 __global__ void __launch_bounds__(kKnnThreads) knn_cov_kernel(GridView g, int lo, int hi, int k,
                                                                double* __restrict__ normals,

@@ -24,8 +24,6 @@ namespace gicpb {
 namespace {
 
 constexpr int kNnThreads = 128;
-constexpr int kQueueCap = 10;  // point ranges a thread can queue before it scans (3x3 rows, one of them split by a brick edge); 16 entries took
-                               // 16 KB of every block from L1: correspondence kernels of a job 1.616 -> 1.58 ms at 1 M, 27.5 -> 26.5 ms at 8 M
 
 // gate2 >= 0: only candidates with d2 < gate2 count (gate2 == 0 admits none, as PCL's `nn_dists[0] < dist_threshold`
 // with a zero threshold); gate2 < 0: ungated
@@ -52,7 +50,7 @@ __device__ __forceinline__ bool search_item(const GridView& g, float qx, float q
     hit = nn_far<kEarlyExit>(g, q, s);
     return true;
   }
-  const int r = nn_near<kEarlyExit, kNnThreads, kQueueCap>(g, q, s, qb, qe, fw.near_rings);
+  const int r = nn_near<kEarlyExit, kNnThreads, kNnQueueCap>(g, q, s, qb, qe, fw.near_rings);
   if (r == kNear_Far) {
     fw.flags[item] = 1;
     return false;
@@ -62,8 +60,8 @@ __device__ __forceinline__ bool search_item(const GridView& g, float qx, float q
 }
 
 #define GICPB_NEAR_QUEUE()                                     \
-  __shared__ unsigned s_qb[kFar ? 1 : kQueueCap * kNnThreads]; \
-  __shared__ unsigned s_qe[kFar ? 1 : kQueueCap * kNnThreads]; \
+  __shared__ unsigned s_qb[kFar ? 1 : kNnQueueCap * kNnThreads]; \
+  __shared__ unsigned s_qe[kFar ? 1 : kNnQueueCap * kNnThreads]; \
   unsigned* qb = s_qb + (kFar ? 0 : threadIdx.x);              \
   unsigned* qe = s_qe + (kFar ? 0 : threadIdx.x)
 
@@ -327,7 +325,7 @@ __global__ void __launch_bounds__(kNnThreads, kFar ? 4 : 6) resolution_kernel(Gr
     const Query q = make_query(g, p.x, p.y, p.z);
     if (kFar) {
       knn_far(g, q, L);
-    } else if (!knn_near<kNnThreads, kQueueCap>(g, q, L, qb, qe)) {
+    } else if (!knn_near<kNnThreads, kNnQueueCap>(g, q, L, qb, qe)) {
       fw.flags[i] = 1;
       return;
     }

@@ -192,6 +192,9 @@ static void brute_nn(const HostIndex& ix, float qx, float qy, float qz, NNState&
   }
 }
 
+// kCap: the queue length of the near searches (QueueVisitor).  The library's own caps (common.cuh), or 1, which sends every
+// range through the overflow path (drain before the next range is queued).
+template <int kCap>
 static void check_nn(const HostIndex& ix, float qx, float qy, float qz, float gate2, int seed_pos, const char* what) {
   NNState a, b;
   if (gate2 > 0) { a.best = gate2; a.pos = -1; a.oi = -1; } else { a.best = inf(); a.pos = -1; a.oi = INT_MAX; }
@@ -202,9 +205,9 @@ static void check_nn(const HostIndex& ix, float qx, float qy, float qz, float ga
     if (cand_less(d, oi, a.best, a.oi)) { a.best = d; a.pos = seed_pos; a.oi = oi; }
   }
   const NNState a0 = a;
-  unsigned qb[16], qe[16];
+  unsigned qb[kCap], qe[kCap];
   const Query q = make_query(ix.g, qx, qy, qz);
-  const int near = nn_near<false, 1, 16>(ix.g, q, a, qb, qe);
+  const int near = nn_near<false, 1, kCap>(ix.g, q, a, qb, qe);
   if (near == kNear_Far) { a = a0; nn_far<false>(ix.g, q, a); ++g_far; }
   if (mode_far_only) { a = a0; nn_far<false>(ix.g, q, a); }
   brute_nn(ix, qx, qy, qz, b);
@@ -218,7 +221,7 @@ static void check_nn(const HostIndex& ix, float qx, float qy, float qz, float ga
   if (gate2 > 0) {
     NNState e; e.best = gate2; e.pos = -1; e.oi = -1;
     const NNState e0 = e;
-    const int r = nn_near<true, 1, 16>(ix.g, q, e, qb, qe);
+    const int r = nn_near<true, 1, kCap>(ix.g, q, e, qb, qe);
     bool hit = r == kNear_Stop;
     if (r == kNear_Far) { e = e0; hit = nn_far<true>(ix.g, q, e); }
     ++g_checks;
@@ -226,15 +229,16 @@ static void check_nn(const HostIndex& ix, float qx, float qy, float qz, float ga
   }
 }
 
+template <int kCap>
 static void check_knn(const HostIndex& ix, int i, int k) {
   std::vector<unsigned long long> lk(k);
   KnnVisitor<1> v;
   v.pts = ix.pts.data(); v.lkey = lk.data(); v.k = k;
   const float4 q = ix.pts[i];
   v.qx = q.x; v.qy = q.y; v.qz = q.z;
-  unsigned qb[16], qe[16];
+  unsigned qb[kCap], qe[kCap];
   const Query qq = make_query(ix.g, q.x, q.y, q.z);
-  if (mode_far_only || !knn_near<1, 12>(ix.g, qq, v, qb, qe)) { knn_far(ix.g, qq, v); ++g_knn_far; }
+  if (mode_far_only || !knn_near<1, kCap>(ix.g, qq, v, qb, qe)) { knn_far(ix.g, qq, v); ++g_knn_far; }
   std::vector<std::pair<std::pair<float, int>, int>> all(ix.g.n);
   for (int j = 0; j < ix.g.n; ++j) all[j] = {{dist2(q.x, q.y, q.z, ix.pts[j]), f2i_bits(ix.pts[j].w)}, j};
   const int kk = std::min(k, ix.g.n);
@@ -245,12 +249,35 @@ static void check_knn(const HostIndex& ix, int i, int k) {
   if (!ok) { if (g_fail < 10) printf("kNN mismatch at sorted point %d (count %d)\n", i, v.count); ++g_fail; }
 }
 
+// Every point set of run() is moved by offset * (1, -0.5, 0.25): far from the origin the grid margin (4e-6 |x|) widens and
+// the near searches hand more queries to the far traversal.
+template <int kNnCap, int kKnnCap>
+static void run(float offset);
+
 int main(int argc, char** argv) {
-  mode_far_only = argc > 1 && std::string(argv[1]) == "far";  // answer every query with the hierarchical traversal alone
+  // far: answer every query with the hierarchical traversal alone; cap1: queues of one entry; offset=X: see run()
+  bool cap1 = false;
+  float offset = 0.f;
+  for (int a = 1; a < argc; ++a) {
+    const std::string s = argv[a];
+    if (s == "far") mode_far_only = true;
+    else if (s == "cap1") cap1 = true;
+    else if (s.rfind("offset=", 0) == 0) offset = std::strtof(s.c_str() + 7, nullptr);
+    else { printf("unknown argument %s\n", s.c_str()); return 2; }
+  }
+  if (cap1) run<1, 1>(offset);
+  else run<kNnQueueCap, kKnnQueueCap>(offset);
+  printf("%ld checks, %ld failures (%ld NN and %ld kNN queries went through the far traversal)\n", g_checks, g_fail, g_far,
+         g_knn_far);
+  return g_fail ? 1 : 0;
+}
+
+template <int kNnCap, int kKnnCap>
+static void run(float offset) {
   std::mt19937 rng(12345);
   std::uniform_real_distribution<float> U(0.f, 1.f);
   std::normal_distribution<float> N(0.f, 1.f);
-  for (int scenario = 0; scenario < 9; ++scenario) {
+  for (int scenario = 0; scenario < 10; ++scenario) {
     std::vector<float3> pts;
     float h = 0.05f;
     const char* name = "";
@@ -296,6 +323,11 @@ int main(int argc, char** argv) {
         pts.push_back({a, b, (i & 1 ? 0.06f : 0.0f) + (a > 1.0f ? 0.15f : 0.0f) + 0.0005f * N(rng)});
       }
       h = 0.02f;
+    } else if (scenario == 9) {  // lattice of spacing 2^-6 on cells of that edge, points one float either side of the faces
+      name = "face ulps";
+      for (int x = 0; x < 16; ++x) for (int y = 0; y < 16; ++y) for (int z = 0; z < 16; ++z)
+        pts.push_back({0.015625f * x, 0.015625f * y, 0.015625f * z});
+      h = 0.015625f;
     } else {  // cube faces (reference fixture shape), coarse cells
       name = "cube";
       for (int i = 0; i < 5000; ++i) {
@@ -305,6 +337,17 @@ int main(int argc, char** argv) {
       }
       h = 0.12f;
     }
+    for (auto& p : pts) {
+      p.x += offset;
+      p.y -= 0.5f * offset;
+      p.z += 0.25f * offset;
+    }
+    if (scenario == 9)  // after the offset: one float of the coordinate where it is, in turn up, down or not at all
+      for (size_t i = 0; i < pts.size(); ++i) {
+        float* c = (i / 3) % 3 == 0 ? &pts[i].x : ((i / 3) % 3 == 1 ? &pts[i].y : &pts[i].z);
+        if (i % 3 == 1) *c = std::nextafter(*c, INFINITY);
+        if (i % 3 == 2) *c = std::nextafter(*c, -INFINITY);
+      }
     HostIndex ix;
     build_index(pts, h, ix);
     const GridView& g = ix.g;
@@ -320,20 +363,17 @@ int main(int argc, char** argv) {
       else if (mode == 3) { qx = g.ox + ext * (3 * U(rng) - 1); qy = g.oy + ext * (3 * U(rng) - 1); qz = g.oz + ext * (3 * U(rng) - 1); }  // anywhere, also outside
       else if (mode == 4) { qx = p.x; qy = p.y; qz = p.z; }                                                               // exactly on a point
       else { qx = p.x + 0.5f * h; qy = p.y; qz = p.z; }
-      check_nn(ix, qx, qy, qz, 0.f, -1, name);
-      check_nn(ix, qx, qy, qz, (2.5f * h) * (2.5f * h), -1, name);
-      check_nn(ix, qx, qy, qz, (60.f * h) * (60.f * h), -1, name);
-      check_nn(ix, qx, qy, qz, 0.f, (int)(rng() % pts.size()), name);           // random (bad) seed
-      check_nn(ix, qx, qy, qz, (60.f * h) * (60.f * h), (int)(rng() % pts.size()), name);
+      check_nn<kNnCap>(ix, qx, qy, qz, 0.f, -1, name);
+      check_nn<kNnCap>(ix, qx, qy, qz, (2.5f * h) * (2.5f * h), -1, name);
+      check_nn<kNnCap>(ix, qx, qy, qz, (60.f * h) * (60.f * h), -1, name);
+      check_nn<kNnCap>(ix, qx, qy, qz, 0.f, (int)(rng() % pts.size()), name);           // random (bad) seed
+      check_nn<kNnCap>(ix, qx, qy, qz, (60.f * h) * (60.f * h), (int)(rng() % pts.size()), name);
     }
-    const int k = std::min(20, (int)pts.size());
-    for (int t = 0; t < 1500; ++t) check_knn(ix, (int)(rng() % pts.size()), k);
-    for (int t = 0; t < 200; ++t) check_knn(ix, (int)(rng() % pts.size()), 2);
-    for (int t = 0; t < 200; ++t) check_knn(ix, (int)(rng() % pts.size()), std::min(32, (int)pts.size()));
+    const int n = (int)pts.size();
+    for (int t = 0; t < 1500; ++t) check_knn<kKnnCap>(ix, (int)(rng() % pts.size()), std::min(20, n));
+    for (const int k : {2, 3, 31, 32})
+      for (int t = 0; t < 200; ++t) check_knn<kKnnCap>(ix, (int)(rng() % pts.size()), std::min(k, n));
     printf("scenario %-12s n=%6d grid %dx%dx%d bricks %dx%dx%d: %s\n", name, g.n, g.nx, g.ny, g.nz, g.nbx, g.nby, g.nbz,
            g_fail == fail0 ? "ok" : "FAILED");
   }
-  printf("%ld checks, %ld failures (%ld NN and %ld kNN queries went through the far traversal)\n", g_checks, g_fail, g_far,
-         g_knn_far);
-  return g_fail ? 1 : 0;
 }
