@@ -59,7 +59,6 @@ typedef struct gicpb_params {
   float points_per_cell;          /* density target when cell_size <= 0                       (6.0)   */
   int mahalanobis_fp32;           /* 0: store M as 6 doubles (default); 1: 6 floats (56 B/pair cost pass) */
   int use_previous_match;         /* 1 (default): seed each NN search with last iteration's match     */
-  int l2_persist;                 /* 1 (default): persisting-L2 window on the per-pair Mahalanobis array    */
   int cost_moments;               /* 0 (default): one cost-kernel pass over all pairs per evaluation, T*p rounded to
                                    * float exactly as PCL does: the BFGS path is PCL's step for step.
                                    * 1: one pass per OUTER iteration reduces the pairs to the 74 second-order moments

@@ -35,7 +35,6 @@ class Params(ctypes.Structure):
         ("points_per_cell", ctypes.c_float),
         ("mahalanobis_fp32", ctypes.c_int),
         ("use_previous_match", ctypes.c_int),
-        ("l2_persist", ctypes.c_int),
         ("cost_moments", ctypes.c_int),
         ("cost_persistent", ctypes.c_int),
     ]

@@ -652,44 +652,18 @@ void launch_persistent_v(const float4* src, int lo, int n, const float4* pair_tg
 
 // block shape of the resident kernel: 512 threads x 2 stages keeps 80 KB in flight per SM and parks 26 % of 1 M pairs;
 // from 2 M pairs on - where an evaluation is the stream from L2 / HBM and little else - a third stage (120 KB in flight) is
-// worth the pairs it unparks (4 M pairs: 56 -> 51 us per evaluation; 1 M: 13.7 us either way).  GICPB_COST_VARIANT fixes the
-// shape for measurements: 0: 512 x 2, 1: 256 x 3 (60 KB, 30 %), 2: 256 x 2 (40 KB, 34 %), 3: 512 x 3, 4: 512 x 4
-int persistent_variant(int n) {
-  static int v = -2;
-  if (v == -2) {
-    const char* e = std::getenv("GICPB_COST_VARIANT");
-    v = e && *e ? std::atoi(e) : -1;
-    if (v < -1 || v > 4) v = -1;
-  }
-  return v >= 0 ? v : (n >= 2000000 ? 3 : 0);
-}
-
+// worth the pairs it unparks (4 M pairs: 56 -> 51 us per evaluation; 1 M: 13.7 us either way).
 template <typename MT, bool kPeer>
 void launch_persistent_t(const float4* src, int lo, int n, const float4* pair_tgt, const void* maha, const CostCommand* hcmd,
                          CostCommand* dcmd, unsigned epoch, double* partials, unsigned* ticket, double* out,
                          const PeerReduce& pr, unsigned long long idle_ns, int blocks, int smem_optin, cudaStream_t stream,
                          CostPersistentShape* shape) {
-  switch (persistent_variant(n)) {
-    case 1:
-      launch_persistent_v<MT, kPeer, 256, 3>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream, shape);
-      break;
-    case 2:
-      launch_persistent_v<MT, kPeer, 256, 2>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream, shape);
-      break;
-    case 3:
-      launch_persistent_v<MT, kPeer, 512, 3>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream, shape);
-      break;
-    case 4:
-      launch_persistent_v<MT, kPeer, 512, 4>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream, shape);
-      break;
-    default:
-      launch_persistent_v<MT, kPeer, 512, 2>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
-                                             blocks, smem_optin, stream, shape);
-  }
+  if (n >= 2000000)
+    launch_persistent_v<MT, kPeer, 512, 3>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
+                                           blocks, smem_optin, stream, shape);
+  else
+    launch_persistent_v<MT, kPeer, 512, 2>(src, lo, n, pair_tgt, maha, hcmd, dcmd, epoch, partials, ticket, out, pr, idle_ns,
+                                           blocks, smem_optin, stream, shape);
 }
 }  // namespace
 

@@ -209,7 +209,6 @@ struct LocalGroup {
 struct gicpb_ctx {
   int device = 0;
   int num_sms = 148;
-  size_t l2_persist_bytes = 0, l2_window_max = 0;
   cudaStream_t stream = nullptr;
   cudaStream_t copy_stream = nullptr;  // uploads started by gicpb_prefetch_cloud run here, beside the compute stream
   cudaStream_t aux_stream = nullptr;   // gicpb_set_clouds: target covariances beside the source index build
@@ -222,8 +221,8 @@ struct gicpb_ctx {
     int64_t dev_stride = 0;  // stride of the device copy (12 when the cloud went through the packed staged upload)
     cudaEvent_t done = nullptr;
     bool pending = false;
-    bool sharded = false;    // only this rank's slice of the rows was uploaded: take_prefetch gathers the other ranks'
-    bool gathered = false;   // ... unless do_prefetch already did, on the copy stream (one process per GPU)
+    bool sharded = false;    // only this rank's slice of the rows was uploaded: the other ranks' are gathered by do_prefetch
+                             // on the copy stream (one process per GPU) or by take_prefetch (in-process group)
     int64_t chunk_rows = 0;  // rows per rank in the gathered buffer (the last rank's slice may be shorter, or empty)
   } prefetch[4];  // 0 target, 1 source, 2 subtract, 3 difference input (gicpb_group_cloud_difference)
   gicpb_params prm{};
@@ -393,16 +392,6 @@ void update_shard(gicpb_ctx* c) {
   }
 }
 
-// Sharded jobs index only the rank's window of the source (GridIndex::build, world > 1); GICPB_WINDOWED_SOURCE=0: the whole
-// source on every rank, as for the target.
-int source_world(const gicpb_ctx* c) {
-  static const bool enabled = [] {
-    const char* e = std::getenv("GICPB_WINDOWED_SOURCE");
-    return !(e && *e == '0');
-  }();
-  return enabled ? c->world : 1;
-}
-
 // Target covariances are needed in full on every rank, but each is a function of the target cloud alone: every rank
 // computes one contiguous chunk of the (identically sorted) target (start_target_cov, on `knn_stream`) and the chunks
 // are all-gathered in place (finish_covariances, on the context's stream).
@@ -504,18 +493,6 @@ void ensure_pair_buffers(gicpb_ctx* c) {
   c->d_sums.reserve(16);
   c->mom_partials.reserve((size_t)c->num_sms * 80);
   c->d_mom.reserve(80);
-  // The pair arrays are re-read by every cost evaluation of an outer iteration (tens of passes over the same bytes):
-  // ask L2 to keep as much of the Mahalanobis array as its persisting carve-out holds.
-  if (c->l2_persist_bytes > 0 && c->prm.l2_persist != 0 && c->prm.cost_moments == 0) {
-    const size_t bytes = 6 * ns * (c->prm.mahalanobis_fp32 ? sizeof(float) : sizeof(double));
-    cudaStreamAttrValue attr{};
-    attr.accessPolicyWindow.base_ptr = c->maha.get();
-    attr.accessPolicyWindow.num_bytes = std::min(bytes, c->l2_window_max);
-    attr.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)c->l2_persist_bytes / (double)std::max<size_t>(bytes, 1));
-    attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-    GICPB_CUDA(cudaStreamSetAttribute(c->stream, cudaStreamAttributeAccessPolicyWindow, &attr));
-  }
 }
 
 // one correspondence pass under transform T (row-major 4x4 float)
@@ -891,35 +868,22 @@ bool shard_uploads(const gicpb_ctx* c) {
   return enabled && c->world > 1 && (c->local != nullptr || c->comm != nullptr);
 }
 
-// GICPB_GATHER_ON_COPY_STREAM=0: exchange the slices on the compute stream when the cloud is set (measurements)
-bool gather_on_copy_stream() {
-  static const bool enabled = [] {
-    const char* e = std::getenv("GICPB_GATHER_ON_COPY_STREAM");
-    return !(e && *e == '0');
-  }();
-  return enabled;
-}
-
+// in-process group: the other members' slices are copied over from their staging buffers when the cloud is set
 void gather_slices(gicpb_ctx* c, int which) {
   gicpb_ctx::Prefetch& p = c->prefetch[which];
   const size_t chunk_bytes = (size_t)p.chunk_rows * 12;
-  if (c->local) {
-    GICPB_CUDA(cudaStreamSynchronize(c->stream));  // this rank's slice is in place (the stream waits for the copy stream)
-    c->local->barrier();
-    for (int r = 0; r < c->world; ++r) {
-      if (r == c->rank) continue;
-      const int64_t lo = std::min<int64_t>(p.n, (int64_t)r * p.chunk_rows), hi = std::min<int64_t>(p.n, lo + p.chunk_rows);
-      if (hi <= lo) continue;
-      const gicpb_ctx* o = c->local->members[(size_t)r];
-      GICPB_CUDA(cudaMemcpyPeerAsync(p.dev + (size_t)r * chunk_bytes, c->device, o->prefetch[which].dev + (size_t)r * chunk_bytes,
-                                     o->device, (size_t)(hi - lo) * 12, c->stream));
-    }
-    GICPB_CUDA(cudaStreamSynchronize(c->stream));
-    c->local->barrier();  // every rank has what it needs from the others' staging buffers
-  } else {
-    check_nccl(c, c->nccl->AllGather(p.dev + (size_t)c->rank * chunk_bytes, p.dev, chunk_bytes, /*ncclInt8*/ 0, c->comm, c->stream),
-               "ncclAllGather");
+  GICPB_CUDA(cudaStreamSynchronize(c->stream));  // this rank's slice is in place (the stream waits for the copy stream)
+  c->local->barrier();
+  for (int r = 0; r < c->world; ++r) {
+    if (r == c->rank) continue;
+    const int64_t lo = std::min<int64_t>(p.n, (int64_t)r * p.chunk_rows), hi = std::min<int64_t>(p.n, lo + p.chunk_rows);
+    if (hi <= lo) continue;
+    const gicpb_ctx* o = c->local->members[(size_t)r];
+    GICPB_CUDA(cudaMemcpyPeerAsync(p.dev + (size_t)r * chunk_bytes, c->device, o->prefetch[which].dev + (size_t)r * chunk_bytes,
+                                   o->device, (size_t)(hi - lo) * 12, c->stream));
   }
+  GICPB_CUDA(cudaStreamSynchronize(c->stream));
+  c->local->barrier();  // every rank has what it needs from the others' staging buffers
 }
 
 // starts the upload of a host cloud on the copy stream (gicpb_prefetch_cloud)
@@ -960,13 +924,11 @@ void do_prefetch(gicpb_ctx* c, int which, const void* xyz, int64_t n, int64_t st
       GICPB_CUDA(cudaMemcpyAsync(p.dev, xyz, (size_t)(n - 1) * stride + 12, cudaMemcpyHostToDevice, c->copy_stream));
     }
   }
-  p.gathered = false;
-  if (p.sharded && !c->local && gather_on_copy_stream()) {
+  if (p.sharded && !c->local) {
     // one process per GPU: the slices are exchanged on the copy stream as soon as this rank's has arrived - for the source
     // that is WHILE the target is indexed on the compute stream, not in front of the source's own index build
     check_nccl(c, c->nccl->AllGather(p.dev + (size_t)c->rank * (size_t)p.chunk_rows * 12, p.dev, (size_t)p.chunk_rows * 12,
                                      /*ncclInt8*/ 0, c->comm, c->copy_stream), "ncclAllGather");
-    p.gathered = true;
   }
   GICPB_CUDA(cudaEventRecord(p.done, c->copy_stream));
   p.host = xyz;
@@ -987,7 +949,7 @@ bool take_prefetch(gicpb_ctx* c, int which, const void* xyz, int64_t n, int64_t 
   if (!p.pending) return false;
   p.pending = false;
   GICPB_CUDA(cudaStreamWaitEvent(c->stream, p.done, 0));
-  if (p.sharded && !p.gathered) gather_slices(c, which);
+  if (p.sharded && c->local) gather_slices(c, which);
   return true;
 }
 
@@ -1249,7 +1211,6 @@ void gicpb_default_params(gicpb_params* p) {
   p->points_per_cell = 6.0f;
   p->mahalanobis_fp32 = 0;
   p->use_previous_match = 1;
-  p->l2_persist = 1;
   p->cost_moments = 0;
   p->cost_persistent = 1;
   // GICPB_COST_PERSISTENT=0: one launch per evaluation (for runs under a profiler, which serialises launches and keeps the
@@ -1273,18 +1234,6 @@ int gicpb_create(int device, gicpb_ctx** out) {
     if (prop.major < 10) throw CudaError("libgicp_b200 is built for sm_100a only; found sm_" +
                                          std::to_string(prop.major) + std::to_string(prop.minor));
     c->num_sms = prop.multiProcessorCount;
-    // A persisting L2 carve-out for the Mahalanobis array is opt-in (GICPB_L2_PERSIST=1): reserved for the lifetime of the
-    // context it takes 79 of the 126 MB away from everything else - reorder_kernel of an 8 M-point index build ran 0.97 ms
-    // with it and 0.35 ms without - while the evaluations, which keep a quarter of the pairs in shared memory, gain nothing
-    // measurable from it (align 38.57 vs 38.43 ms at 8 M, 2.994 vs 2.996 ms at 1 M).
-    const char* l2env = std::getenv("GICPB_L2_PERSIST");
-    const bool l2_wanted = l2env && *l2env == '1';
-    if (l2_wanted && prop.persistingL2CacheMaxSize > 0 &&
-        cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)prop.persistingL2CacheMaxSize) == cudaSuccess) {
-      c->l2_persist_bytes = (size_t)prop.persistingL2CacheMaxSize;
-      c->l2_window_max = (size_t)prop.accessPolicyMaxWindowSize;
-    }
-    cudaGetLastError();
     GICPB_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     {
       // gicpb_set_clouds runs the target's covariance pass on aux_stream beside the source's index build on the main
@@ -1513,7 +1462,7 @@ int gicpb_set_source(gicpb_ctx* c, const void* xyz, int64_t n, int64_t stride, i
       on_device = 1;
     }
     c->src.build(xyz, n, stride, on_device != 0, c->prm.cell_size, c->prm.points_per_cell, c->stream, &c->stager, c->rank,
-                 source_world(c));
+                 c->world);
     update_shard(c);
   });
 }
@@ -1550,7 +1499,7 @@ int gicpb_set_clouds(gicpb_ctx* c, const void* target, int64_t n_target, int64_t
         s_dev = 1;
       }
       c->src.build(source, n_source, source_stride, s_dev != 0, c->prm.cell_size, c->prm.points_per_cell, c->stream, &c->stager,
-                   c->rank, source_world(c));
+                   c->rank, c->world);
     } catch (...) {
       if (overlap) cudaStreamSynchronize(c->aux_stream);  // nothing may still be running on the target when we leave
       throw;

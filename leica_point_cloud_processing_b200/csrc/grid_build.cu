@@ -398,15 +398,6 @@ struct BuildTrace {
 
 inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
 
-// GICPB_SB_PLANE=0 leaves the superbrick slabs out of the view (measurements)
-inline bool use_sb_plane() {
-  static const bool on = [] {
-    const char* e = std::getenv("GICPB_SB_PLANE");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
 }  // namespace
 
 // Oriented slab of every occupied brick (GridView::brick_plane, used by visit_brick): one warp per brick slot.  The
@@ -1017,7 +1008,7 @@ void GridIndex::index_points(const float4* pts, int64_t n, int64_t n_valid, cons
   brick_plane_kernel<<<blocks_for(n_slots * 32, 128), 128, 0, stream>>>(pts_sorted_.get(), cell_start_.get(), (int)n_slots,
                                                                         brick_plane_.get());
   GICPB_LAUNCHED();
-  if (far_queries_ && use_sb_plane()) {
+  if (far_queries_) {
     sb_plane_.reserve(n_sb * 5);
     GridView gv = g;  // the kernel needs the geometry and the brick numbering only
     sb_plane_kernel<<<(unsigned)n_sb, kSbThreads, 0, stream>>>(gv, pts_sorted_.get(), cell_start_.get(), brick_slot_.get(), sb_mask_.get(),
@@ -1030,7 +1021,7 @@ void GridIndex::index_points(const float4* pts, int64_t n, int64_t n_valid, cons
 
   g.pts = pts_sorted_.get();
   g.brick_plane = brick_plane_.get();
-  g.sb_plane = (far_queries_ && use_sb_plane()) ? sb_plane_.get() : nullptr;
+  g.sb_plane = far_queries_ ? sb_plane_.get() : nullptr;
   g.brick_slot = brick_slot_.get();
   g.cell_start = cell_start_.get();
   g.pos_of = pos_of_.get();

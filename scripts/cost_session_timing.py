@@ -1,6 +1,6 @@
 """Wall time of one cost / gradient evaluation as the BFGS loop sees it: the resident kernel of an inner solve
 (cost_persistent=1, bench hook 4) against one launch per evaluation (hook 5), the bare kernel (hook 1), and the whole job
-both ways.  GICPB_COST_VARIANT selects the block shape of the resident kernel.
+both ways, with the block shape (threads x ring stages) the resident kernel took.
 Usage: python scripts/cost_session_timing.py [points ...]"""
 import os
 import sys
@@ -30,8 +30,9 @@ for n in sizes:
     ms_res, _ = eng.bench_kernel(4, T, iters=200)
     ms_one, _ = eng.bench_kernel(5, T, iters=200)
     ms_k, _ = eng.bench_kernel(1, T, iters=50)
+    _, _, info = eng.cost_session(np.zeros((1, 6)))
     same = np.array_equal(out[0][1]["transform"], out[1][1]["transform"])
-    print(f"n={n} variant={os.environ.get('GICPB_COST_VARIANT', '0')} eval wall us: resident {1e3 * ms_res:.2f}  per-launch {1e3 * ms_one:.2f}  "
+    print(f"n={n} shape={info['threads']}x{info['stages']} eval wall us: resident {1e3 * ms_res:.2f}  per-launch {1e3 * ms_one:.2f}  "
           f"kernel-only {1e3 * ms_k:.2f} | job ms (host arrays, wall): per-launch {out[0][0]:.3f} resident {out[1][0]:.3f} "
           f"evals {out[1][1]['cost_evaluations']} ms_cost {out[0][1]['ms_cost']:.3f} -> {out[1][1]['ms_cost']:.3f} "
           f"ms_corr {out[1][1]['ms_corr']:.3f} identical={same}", flush=True)

@@ -47,6 +47,26 @@ def test_default_params_match_the_reference(lib):
     assert (p.transformation_epsilon, p.rotation_epsilon, p.max_corr_distance, p.gicp_epsilon) == (4e-3, 2e-3, 4e-2, 1e-3)
 
 
+def test_params_layout_matches_the_header(tmp_path):
+    """_capi.Params is gicpb_params field for field: same names in the same order, same offsets, same size (a field
+    added, removed or moved on one side only would shift every field after it)"""
+    from leica_point_cloud_processing_b200 import Params
+    header = open(os.path.join(ROOT, "include", "gicp_b200.h")).read()
+    body = header[header.index("typedef struct gicpb_params {"):header.index("} gicpb_params;")]
+    fields = re.findall(r"^\s+(?:int|float|double)\s+(\w+);", body, re.M)
+    assert fields == [name for name, _ in Params._fields_]
+    src = tmp_path / "params_layout.cpp"
+    src.write_text("#include <cstddef>\n#include <cstdio>\n#include \"gicp_b200.h\"\nint main() {\n"
+                   "  std::printf(\"sizeof %zu\\n\", sizeof(gicpb_params));\n" +
+                   "".join(f"  std::printf(\"{f} %zu\\n\", offsetof(gicpb_params, {f}));\n" for f in fields) +
+                   "  return 0;\n}\n")
+    exe = str(tmp_path / "params_layout")
+    subprocess.check_call(["g++", "-std=c++14", "-Wall", "-Werror", "-I" + os.path.join(ROOT, "include"), str(src), "-o", exe])
+    c_layout = {k: int(v) for k, v in (line.split() for line in subprocess.check_output([exe], text=True).splitlines())}
+    assert c_layout.pop("sizeof") == ctypes.sizeof(Params)
+    assert c_layout == {f: getattr(Params, f).offset for f in fields}
+
+
 def test_no_cpu_fallback(lib):
     import torch
     from leica_point_cloud_processing_b200 import Engine, GicpError

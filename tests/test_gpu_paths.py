@@ -13,9 +13,6 @@ E. a member of an EngineGroup used on its own: a plain single-GPU context over t
 
 A sum of n terms in double differs from any other order of the same sum by at most n * 2^-53 * sum |terms|: a fitness or cost
 bound derived from that checks every term, where a hand-picked tolerance could hide a wrong neighbour among millions."""
-import os
-import subprocess
-import sys
 import time
 
 import numpy as np
@@ -25,9 +22,8 @@ from leica_point_cloud_processing_b200 import synth
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 U = 2.0 ** -53
-SWITCH = (1_999_999, 2_000_000, 2_000_001)   # far_tile_for / persistent_variant boundary
+SWITCH = (1_999_999, 2_000_000, 2_000_001)   # far_tile_for / resident cost kernel shape boundary
 
 
 def _params(**kw):
@@ -317,59 +313,33 @@ def test_resident_cost_kernel_shapes(eng, fast_oracle, big_cloud, n):
     eng.set_params(**_params())
 
 
-_EDGES = r"""
-import sys
-import numpy as np
-sys.path.insert(0, {root!r})
-sys.path.insert(0, {tests!r})
-from leica_point_cloud_processing_b200 import Engine, synth
-from oracle.oracle import Oracle
-from test_gpu_paths import _check_cost_sessions, _states
-
-orc = Oracle(fast=True)
-e = Engine(0)
-pool = synth.panel_points(600_000, 66, noise_sigma=5e-4)
-
-
-def per_block(n, blocks):
-    return (-(-n // blocks) + 15) & ~15
-
-
-for fp32 in (0, 1):
-    e.set_params(max_corr_distance=0.01, points_per_cell=6.0, mahalanobis_fp32=fp32, cost_persistent=1)
-    probe = pool[:20_000]
-    e.set_clouds(probe, probe)
-    e.correspondences(np.eye(4, dtype=np.float32))
-    _, _, info = e.cost_session(_states(1, 0))
-    B, C = info["blocks"], info["resident_cap"]
-    assert (info["threads"], info["stages"]) == (512, 3) and C % 16 == 0 and C > 0, info
-    # (pairs per block, pairs of the last block): streamed pairs of the last block 0 / 1 / 511 / 512 / 513, and an odd last
-    # block below the resident cap (its bulk copy of 24-byte rows is rounded up to 16 bytes)
-    cases = [(C, C - 1), (C, C // 2 + 1), (C + 16, C + 1), (C + 512, C + 511), (C + 512, C + 512), (C + 528, C + 513)]
-    for per, last in cases:
-        n = (B - 1) * per + last
-        assert per_block(n, B) == per and n <= len(pool), (per, last, n)
-        cloud = pool[:n]
-        e.set_params(cost_persistent=1)
-        e.set_clouds(cloud, cloud)
-        assert e.correspondences(np.eye(4, dtype=np.float32))[0] == n
-        info = _check_cost_sessions(e, orc, cloud, _states(5, n), (512, 3))
-        assert info["pairs_per_block"] == per and info["resident"] == min(per, C)
-        print(f"fp32 {{fp32}} n {{n}}: streamed per block {{per - min(per, C)}}, last block {{last}} pairs "
-              f"({{last - min(last, C)}} streamed)")
-e.close()
-print("edges ok")
-"""
-
-
-def test_resident_cost_kernel_block_edges():
-    """GICPB_COST_VARIANT=3 (512 x 3 at any size; read once per process) at small pair counts chosen from the reported
-    resident cap, so that blocks stream 0, 1, 511, 512 and 513 pairs past what they park"""
-    code = _EDGES.format(root=ROOT, tests=os.path.join(ROOT, "tests"))
-    run = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=900,
-                         env=dict(os.environ, GICPB_COST_VARIANT="3"))
-    print(run.stdout[-4000:], run.stderr[-4000:])
-    assert run.returncode == 0 and "edges ok" in run.stdout
+def test_resident_cost_kernel_block_edges_512x2(eng, fast_oracle):
+    """The 512 x 2 shape (below 2 M pairs) at pair counts chosen from the reported resident cap, so that blocks stream 0, 1,
+    511, 512 and 513 pairs past what they park"""
+    pool = synth.panel_points(600_000, 66, noise_sigma=5e-4)
+    for fp32 in (0, 1):
+        eng.set_params(**_params(max_corr_distance=0.01, mahalanobis_fp32=fp32))
+        probe = pool[:20_000]
+        eng.set_clouds(probe, probe)
+        eng.correspondences(np.eye(4, dtype=np.float32))
+        _, _, info = eng.cost_session(_states(1, 0))
+        B, C = info["blocks"], info["resident_cap"]
+        assert (info["threads"], info["stages"]) == (512, 2) and C % 16 == 0 and C > 0, info
+        # (pairs per block, pairs of the last block): streamed pairs of the last block 0 / 1 / 511 / 512 / 513, and an odd
+        # last block below the resident cap (its bulk copy of 24-byte rows is rounded up to 16 bytes)
+        cases = [(C, C - 1), (C, C // 2 + 1), (C + 16, C + 1), (C + 512, C + 511), (C + 512, C + 512), (C + 528, C + 513)]
+        for per, last in cases:
+            n = (B - 1) * per + last
+            assert ((-(-n // B) + 15) & ~15) == per and n <= len(pool), (per, last, n)
+            cloud = pool[:n]
+            eng.set_params(cost_persistent=1)
+            eng.set_clouds(cloud, cloud)
+            assert eng.correspondences(np.eye(4, dtype=np.float32))[0] == n
+            info = _check_cost_sessions(eng, fast_oracle, cloud, _states(5, n), (512, 2))
+            assert info["pairs_per_block"] == per and info["resident"] == min(per, C)
+            print(f"fp32 {fp32} n {n}: streamed per block {per - min(per, C)}, last block {last} pairs "
+                  f"({last - min(last, C)} streamed)")
+    eng.set_params(**_params())
 
 
 def test_cost_epochs_alternate_across_the_wrap(oracle, cube_pair):

@@ -17,15 +17,12 @@ at the end of a distance shell and inside one, 0 / 1 km / 8 km out), 40 copies o
 covariance is exactly zero; C the cube and the panel 300 m to 10 km out, and points one float either side of the cell
 faces; D the near / far split and neighbourhoods that must cross to another cluster; E non-finite rows and the k limit;
 F k and gicp_epsilon changed on a context that already holds covariances, set_clouds against the separate calls; G a
-1 M-point panel; H the cloud resolution (k = 2) of all three slots; I the 128-thread build of the near kernel.
+1 M-point panel; H the cloud resolution (k = 2) of all three slots.
 
 CPU part (-m "not gpu"): the fixtures are what they claim (complete shells, exact floats, ties kept after the offset,
 exactly zero raw covariances, the finite-subset index map monotone).
 """
 import contextlib
-import os
-import subprocess
-import sys
 import time
 
 import numpy as np
@@ -34,7 +31,6 @@ import pytest
 from _cov_util import normal_error_bound, raw_covariances, regularised_from_svd
 from leica_point_cloud_processing_b200 import synth
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OFFSET_DIR = np.array([1.0, -0.5, 0.25])
 SP = 2.0 ** -6                    # lattice spacing: every coordinate and every d2 of the lattices is an exact float
 SHELLS = [1, 6, 12, 8, 6, 24]     # lattice points at d2 = 0, 1, 2, 3, 4, 5 spacings^2 around an interior point
@@ -582,17 +578,3 @@ def test_resolution(engine, oracle, cube_pair, name):
         assert ref == 0.0 and engine.cloud_resolution(0) == 0.0
     print(f"H {name}: n={len(cloud)} count={cnt} res={ref:.9g} tol={tol:.2e}")
 
-
-# ---- I. the 128-thread near kernel --------------------------------------------------------------------------------------------
-@pytest.mark.gpu
-def test_128_thread_near_kernel_gives_the_same_results():
-    """GICPB_KNN_THREADS=128 builds the near instance with 128-thread blocks (knn_cov.cu, for measurements); it is meant
-    to leave every result unchanged.  A short part of A and C again in a process with it set."""
-    sel = "test_every_k and cube-0.0 or test_far_from_the_origin and cube-10000.0 or test_clump_and_outliers_go_far"
-    env = dict(os.environ, GICPB_KNN_THREADS="128")
-    out = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", "-m", "gpu", "-k", sel,
-                          os.path.abspath(__file__)], cwd=ROOT, env=env, capture_output=True, text=True, timeout=1800)
-    tail = out.stdout[-3000:] + out.stderr[-2000:]
-    assert out.returncode == 0, tail
-    assert " passed" in out.stdout and "failed" not in out.stdout, tail
-    print(out.stdout.strip().splitlines()[-1])
