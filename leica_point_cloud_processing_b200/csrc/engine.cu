@@ -159,6 +159,13 @@ float round_up_to_float(double v) {  // smallest float >= v
   return f;
 }
 
+// the correspondence gate of a max_corr_distance: PCL pairs iff (double)d2 < distance^2, i.e. d2 < the float rounded up;
+// a NaN distance pairs nothing (d2 < NaN is false), as the zero gate does
+float corr_gate2(double max_corr_distance) {
+  const double thr = max_corr_distance * max_corr_distance;
+  return std::isnan(thr) ? 0.f : round_up_to_float(thr);
+}
+
 double now_ms() {
   return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
@@ -503,8 +510,7 @@ void run_correspondences(gicpb_ctx* c, const float* T16, bool first, int near_ri
   RotD R;
   for (int i = 0; i < 3; ++i)
     for (int j = 0; j < 3; ++j) R.m[3 * i + j] = (double)T16[4 * i + j];
-  const double thr = c->prm.max_corr_distance * c->prm.max_corr_distance;
-  const float gate2 = round_up_to_float(thr);
+  const float gate2 = corr_gate2(c->prm.max_corr_distance);
   const bool fp32 = c->prm.mahalanobis_fp32 != 0;
   const bool use_prev = c->prm.use_previous_match != 0 && !first && c->pairs_valid && c->pairs_fp32 == fp32;
   GICPB_CUDA(cudaEventRecord(c->ev0, c->stream));
@@ -954,9 +960,10 @@ bool take_prefetch(gicpb_ctx* c, int which, const void* xyz, int64_t n, int64_t 
 }
 
 // keep iff (double)d2 > thr.  With thr_f = largest float <= thr this is d2 > thr_f, i.e. NOT (d2 < next(thr_f)).
-float difference_thr_next(double thr, bool* always_keep) {
-  *always_keep = thr < 0;
-  if (*always_keep) return 0.f;
+// thr < 0 keeps every finite point and a NaN thr none, without a search (and without a NaN search radius).
+float difference_thr_next(double thr, DiffMode* mode) {
+  *mode = std::isnan(thr) ? kDiffKeepNone : thr < 0 ? kDiffKeepAll : kDiffSearch;
+  if (*mode != kDiffSearch) return 0.f;
   float tf = (float)thr;
   if ((double)tf > thr) tf = std::nextafterf(tf, -INFINITY);
   return std::nextafterf(tf, INFINITY);
@@ -1115,8 +1122,8 @@ void check_difference_args(const void* input, int64_t n_input, int64_t input_str
 unsigned long long group_difference_rank(gicpb_ctx* c, const void* input, int64_t n, int64_t input_stride,
                                          const void* subtract, int64_t n_sub, int64_t sub_stride, double thr,
                                          uint8_t* mask) {
-  bool always_keep = false;
-  const float thr_next = difference_thr_next(thr, &always_keep);
+  DiffMode mode = kDiffSearch;
+  const float thr_next = difference_thr_next(thr, &mode);
   const double radius = std::sqrt((double)thr_next);
   // 1. both clouds: this rank's slice of the rows on the copy stream, the other slices from the other members
   const void* sub_p = subtract;
@@ -1164,10 +1171,10 @@ unsigned long long group_difference_rank(gicpb_ctx* c, const void* input, int64_
                                                 c->route_pos.get(), c->route_tmp.get(), c->stream);
     c->io_b.reserve((size_t)std::max<int64_t>(n_own, 1));
     launch_difference(c->sub.view(), reinterpret_cast<const unsigned char*>(c->queries.get()), n_own, 16, thr_next,
-                      always_keep, c->io_b.get(), c->counter.get(), far_work(c, n_own), c->stream);
+                      mode, c->io_b.get(), c->counter.get(), far_work(c, n_own), c->stream);
     scatter_keep(c->queries.get(), c->io_b.get(), n_own, c->keep_full.get(), c->stream);
   } else {
-    launch_difference(c->sub.view(), d_in + lo * input_stride, len, input_stride, thr_next, always_keep,
+    launch_difference(c->sub.view(), d_in + lo * input_stride, len, input_stride, thr_next, mode,
                       c->keep_full.get() + lo, c->counter.get(), far_work(c, len), c->stream);
   }
   unsigned long long kept = 0;
@@ -1588,10 +1595,9 @@ int gicpb_difference_run(gicpb_ctx* c, const void* input, int64_t n, int64_t str
       d_mask = c->io_b.get();
     }
     GICPB_CUDA(cudaMemsetAsync(c->counter.get(), 0, sizeof(unsigned long long), c->stream));
-    bool always_keep = false;
-    const float thr_next = difference_thr_next(thr, &always_keep);
-    launch_difference(c->sub.view(), d_in, n, stride, thr_next, always_keep, d_mask, c->counter.get(), far_work(c, n),
-                      c->stream);
+    DiffMode mode = kDiffSearch;
+    const float thr_next = difference_thr_next(thr, &mode);
+    launch_difference(c->sub.view(), d_in, n, stride, thr_next, mode, d_mask, c->counter.get(), far_work(c, n), c->stream);
     unsigned long long kept = 0;
     GICPB_CUDA(cudaMemcpyAsync(&kept, c->counter.get(), sizeof(kept), cudaMemcpyDeviceToHost, c->stream));
     if (!mask_on_device) download_bytes(c, mask, d_mask, (size_t)n);
@@ -2085,7 +2091,7 @@ int gicpb_bench_kernel(gicpb_ctx* c, int which, const float transform[16], int i
                     cost_grid_blocks(n, c->num_sms), c->stream);
         GICPB_CUDA(cudaEventRecord(c->ev1, c->stream));
       } else if (which == 2) {
-        const float gate2 = round_up_to_float(c->prm.max_corr_distance * c->prm.max_corr_distance);
+        const float gate2 = corr_gate2(c->prm.max_corr_distance);
         GICPB_CUDA(cudaEventRecord(c->ev0, c->stream));
         launch_nn1(c->tgt.view(), c->src.sorted_points() + c->shard_lo, n, T, gate2,
                    reinterpret_cast<int*>(c->io_b.get()), reinterpret_cast<float*>(c->io_b.get() + (size_t)n * 4), nullptr,

@@ -94,8 +94,11 @@ int fitness_partial_rows(int n, int far_blocks);
 // seed: nullptr, or one sorted-target position (-1 = none) per source point of [lo, hi) as a first candidate
 void launch_fitness(const GridView& g, const float4* src, int lo, int hi, const Rigid& T, double max_range,
                     const int* seed, double* partials, double* out2, const FarWork& fw, cudaStream_t stream);
+// what decides a difference's keep bytes: the search (d2 < thr_next hits), or the threshold alone (thr < 0 keeps every
+// finite point, a NaN threshold none: PCL's `d2 > thr` is then always / never true)
+enum DiffMode : int { kDiffSearch = 0, kDiffKeepAll = 1, kDiffKeepNone = 2 };
 void launch_difference(const GridView& g, const unsigned char* raw, int64_t n, int64_t stride, float thr_next,
-                       bool always_keep, unsigned char* mask, unsigned long long* kept, const FarWork& fw,
+                       DiffMode mode, unsigned char* mask, unsigned long long* kept, const FarWork& fw,
                        cudaStream_t stream);
 // use_covariances branch: the mean 2nd-neighbour distance sums (partials sized like the fitness ones); the normals: normals.cu
 void launch_resolution(const GridView& g, double* partials, double* out2, const FarWork& fw, cudaStream_t stream);

@@ -274,7 +274,7 @@ __global__ void __launch_bounds__(kReduceThreads) reduce_partials_kernel(const d
 template <bool kFar>
 __global__ void __launch_bounds__(kNnThreads, kFar ? 6 : 8) difference_kernel(GridView g, const unsigned char* __restrict__ raw,
                                                                  int64_t n, int64_t stride, float thr_next,
-                                                                 int always_keep, unsigned char* __restrict__ mask,
+                                                                 int mode, unsigned char* __restrict__ mask,
                                                                  unsigned long long* __restrict__ kept, FarWork fw) {
   GICPB_NEAR_QUEUE();
   unsigned mine = 0;
@@ -282,8 +282,8 @@ __global__ void __launch_bounds__(kNnThreads, kFar ? 6 : 8) difference_kernel(Gr
     const float* p = reinterpret_cast<const float*>(raw + (int64_t)i * stride);
     const float x = p[0], y = p[1], z = p[2];
     bool keep = false;
-    if (finite3(x, y, z)) {
-      if (always_keep) {
+    if (finite3(x, y, z) && mode != kDiffKeepNone) {
+      if (mode == kDiffKeepAll) {
         keep = true;  // threshold < 0: every finite point with a neighbour is kept
       } else {
         NNState s;
@@ -455,15 +455,14 @@ void launch_fitness(const GridView& g, const float4* src, int lo, int hi, const 
 }
 
 void launch_difference(const GridView& g, const unsigned char* raw, int64_t n, int64_t stride, float thr_next,
-                       bool always_keep, unsigned char* mask, unsigned long long* kept, const FarWork& fw,
+                       DiffMode mode, unsigned char* mask, unsigned long long* kept, const FarWork& fw,
                        cudaStream_t stream) {
   if (n <= 0) return;
   reset_far(fw, n, stream);
-  difference_kernel<false><<<nblocks(n, kNnThreads), kNnThreads, 0, stream>>>(g, raw, n, stride, thr_next,
-                                                                              always_keep ? 1 : 0, mask, kept, fw);
+  difference_kernel<false><<<nblocks(n, kNnThreads), kNnThreads, 0, stream>>>(g, raw, n, stride, thr_next, mode, mask,
+                                                                              kept, fw);
   GICPB_LAUNCHED();
-  difference_kernel<true><<<fw.far_blocks, kNnThreads, 0, stream>>>(g, raw, n, stride, thr_next, always_keep ? 1 : 0,
-                                                                    mask, kept, fw);
+  difference_kernel<true><<<fw.far_blocks, kNnThreads, 0, stream>>>(g, raw, n, stride, thr_next, mode, mask, kept, fw);
   GICPB_LAUNCHED();
 }
 
