@@ -5,8 +5,6 @@
 // src/GICPAlignment.cpp:86-127): guess = identity, per outer iteration one correspondence pass (kernel) and one
 // BFGS solve (host, optimizer.hpp) whose every evaluation is one cost-kernel launch (+ one NCCL all-reduce of 14
 // doubles when the source is sharded over ranks).
-#include <dlfcn.h>
-
 #include <algorithm>
 #include <atomic>
 #include <chrono>
@@ -14,60 +12,19 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
-#include <condition_variable>
 #include <memory>
-#include <mutex>
 #include <thread>
 
 #include "../../include/gicp_b200.h"
 #include "cloud_io.hpp"
+#include "exchange.hpp"
 #include "kernels.hpp"
 #include "optimizer.hpp"
 
 using namespace gicpb;
 
-// ---- NCCL through dlopen -----------------------------------------------------------------------------------
 namespace {
 
-struct NcclApi {
-  typedef struct ncclComm* comm_t;
-  struct unique_id { char internal[128]; };
-  int (*GetUniqueId)(unique_id*) = nullptr;
-  int (*CommInitRank)(comm_t*, int, unique_id, int) = nullptr;
-  int (*CommDestroy)(comm_t) = nullptr;
-  int (*AllReduce)(const void*, void*, size_t, int, int, comm_t, cudaStream_t) = nullptr;
-  int (*AllGather)(const void*, void*, size_t, int, comm_t, cudaStream_t) = nullptr;
-  const char* (*GetErrorString)(int) = nullptr;
-  void* handle = nullptr;
-};
-
-NcclApi* load_nccl(const char* path, std::string& err) {
-  static NcclApi api;
-  if (api.handle) return &api;
-  const char* name = (path && *path) ? path : "libnccl.so.2";
-  void* h = dlopen(name, RTLD_NOW | RTLD_GLOBAL);
-  if (!h) {
-    err = std::string("dlopen(") + name + ") failed: " + dlerror();
-    return nullptr;
-  }
-  api.GetUniqueId = reinterpret_cast<decltype(api.GetUniqueId)>(dlsym(h, "ncclGetUniqueId"));
-  api.CommInitRank = reinterpret_cast<decltype(api.CommInitRank)>(dlsym(h, "ncclCommInitRank"));
-  api.CommDestroy = reinterpret_cast<decltype(api.CommDestroy)>(dlsym(h, "ncclCommDestroy"));
-  api.AllReduce = reinterpret_cast<decltype(api.AllReduce)>(dlsym(h, "ncclAllReduce"));
-  api.AllGather = reinterpret_cast<decltype(api.AllGather)>(dlsym(h, "ncclAllGather"));
-  api.GetErrorString = reinterpret_cast<decltype(api.GetErrorString)>(dlsym(h, "ncclGetErrorString"));
-  if (!api.GetUniqueId || !api.CommInitRank || !api.CommDestroy || !api.AllReduce || !api.AllGather || !api.GetErrorString) {
-    err = "libnccl is missing a required symbol";
-    return nullptr;
-  }
-  api.handle = h;
-  return &api;
-}
-constexpr int kNcclFloat64 = 8, kNcclSum = 0;
-
-struct NcclError : std::runtime_error {
-  explicit NcclError(const std::string& s) : std::runtime_error(s) {}
-};
 struct AlignStop : std::runtime_error {
   int code;
   AlignStop(int c, const std::string& s) : std::runtime_error(s), code(c) {}
@@ -172,46 +129,6 @@ double now_ms() {
 
 }  // namespace
 
-// ---- the contexts of one gicpb_group (one process, several GPUs): what the ranks share ------------------------------------
-struct gicpb_ctx;
-struct GroupAbort : std::runtime_error {
-  GroupAbort() : std::runtime_error("another GPU of the group failed") {}
-};
-struct LocalGroup {
-  int world = 0;
-  std::vector<gicpb_ctx*> members;
-  std::vector<double> slots;  // [world][80]: small sums on their way through the host
-  std::mutex mu;
-  std::condition_variable cv;
-  int waiting = 0;
-  unsigned generation = 0;
-  bool failed = false;
-  // every rank's thread arrives; throws on all of them once one rank has failed (so nobody waits for ever)
-  void barrier() {
-    std::unique_lock<std::mutex> lk(mu);
-    if (failed) throw GroupAbort();
-    const unsigned gen = generation;
-    if (++waiting == world) {
-      waiting = 0;
-      ++generation;
-      cv.notify_all();
-      return;
-    }
-    cv.wait(lk, [&] { return generation != gen || failed; });
-    if (generation == gen) throw GroupAbort();
-  }
-  void fail() {
-    std::lock_guard<std::mutex> lk(mu);
-    failed = true;
-    cv.notify_all();
-  }
-  void reset() {
-    std::lock_guard<std::mutex> lk(mu);
-    failed = false;
-    waiting = 0;
-  }
-};
-
 // ---- context ------------------------------------------------------------------------------------------------
 struct gicpb_ctx {
   int device = 0;
@@ -239,7 +156,6 @@ struct gicpb_ctx {
   VoxelGrid voxel;
   DevBuf<int> uf_parent, uf_root;
   bool cov_ready = false;
-  bool tgt_normals_gathered = false;  // start_target_cov has already exchanged the target's normal chunks (second stream)
   int shard_lo = 0, shard_hi = 0;
   DevBuf<double> n_tgt, n_src;
   DevBuf<int> pair_pos;
@@ -280,21 +196,27 @@ struct gicpb_ctx {
   DevBuf<uint32_t> route_flags, route_pos, route_tmp;
   DevBuf<unsigned char> keep_full, keep_parts;
 
-  NcclApi* nccl = nullptr;
-  NcclApi::comm_t comm = nullptr;
-  int rank = 0, world = 1;
-  LocalGroup* local = nullptr;  // member of a gicpb_group: the collectives go over peer copies / the host, not NCCL
-  bool peer_ipc = false;        // peer.peers[] are cudaIpc mappings (closed on destroy)
-  // fused cost + cross-GPU sum over peer memory (kernels.hpp PeerReduce); falls back to ncclAllReduce when not set up
-  PeerSlots* peer_own = nullptr;
-  PeerReduce peer{};
-  bool peer_ready = false;
+  Exchange ex;                  // who the ranks are and how they exchange data (exchange.hpp)
+  gicpb_group* group = nullptr;  // the group this context is a member of (gicpb_group_create)
 
   // accounting
   double ms_corr = 0, ms_cost = 0;
   int64_t far_queries = 0;
   int64_t cost_evals = 0;
   int64_t window_widened = 0;  // times a sharded source had to be indexed whole after all (GridIndex::widen)
+};
+
+// ---- one process, several GPUs (include/gicp_b200.h "gicpb_group") ------------------------------------------------------
+// The reference's consumer builds its GICPAlignment inside ONE process (reference src/LeicaStateMachine.cpp:138-171), so the
+// multi-GPU path must be reachable without a launcher: a group owns one context per device, every group call runs the same
+// per-rank call on all of them from one host thread per GPU (exactly what the ranks of a torchrun job do, optimisers in lock
+// step), and the collectives stay inside the process: target covariances by peer copies, the 14 cost sums fused into the cost
+// kernel over peer memory (kernels.hpp PeerReduce) when every pair of devices can map each other, else through the host.
+struct gicpb_group {
+  LocalGroup lg;
+  std::vector<gicpb_ctx*> ctx;
+  std::string err;
+  bool fused = false;
 };
 
 namespace {
@@ -330,44 +252,10 @@ int guarded(gicpb_ctx* ctx, F&& fn) {
   } catch (const AlignStop& e) {
     ctx->err = e.what();
     return e.code;
-  } catch (const GroupAbort& e) {
-    ctx->err = e.what();
-    return GICPB_E_STATE;
   } catch (const std::exception& e) {
     ctx->err = e.what();
     return GICPB_E_CUDA;
   }
-}
-
-void check_nccl(gicpb_ctx* c, int rc, const char* what) {
-  if (rc != 0) throw NcclError(std::string(what) + ": " + c->nccl->GetErrorString(rc));
-}
-
-// in-process group: `count` (<= 80) doubles of every rank through the host, added in rank order on every rank (identical sums)
-void local_all_reduce(gicpb_ctx* c, double* dev, int count) {
-  LocalGroup* lg = c->local;
-  double* mine = lg->slots.data() + 80 * (size_t)c->rank;
-  GICPB_CUDA(cudaMemcpyAsync(mine, dev, (size_t)count * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-  GICPB_CUDA(cudaStreamSynchronize(c->stream));
-  lg->barrier();
-  double sum[80];
-  for (int k = 0; k < count; ++k) {
-    double v = 0.0;
-    for (int r = 0; r < lg->world; ++r) v += lg->slots[80 * (size_t)r + k];
-    sum[k] = v;
-  }
-  lg->barrier();  // everybody has read the slots: they may be written again
-  GICPB_CUDA(cudaMemcpyAsync(dev, sum, (size_t)count * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-  GICPB_CUDA(cudaStreamSynchronize(c->stream));
-}
-
-void all_reduce_sum(gicpb_ctx* c, double* dev, int count) {
-  if (c->world <= 1) return;
-  if (c->local) {
-    local_all_reduce(c, dev, count);
-    return;
-  }
-  check_nccl(c, c->nccl->AllReduce(dev, dev, (size_t)count, kNcclFloat64, kNcclSum, c->comm, c->stream), "ncclAllReduce");
 }
 
 constexpr int kFarBlocksPerSm = 6;
@@ -384,14 +272,14 @@ FarWork far_work(gicpb_ctx* c, int64_t n_items, int near_rings = kNearMaxRing) {
 // planes again.  Covariances and pairs belong to one shard: they are dropped whenever the shard changes.
 void update_shard(gicpb_ctx* c) {
   const int lo = c->shard_lo, hi = c->shard_hi;
-  if (c->world == 1 && c->src.ready() && c->src.windowed()) c->src.widen(c->stream);
-  if (c->world > 1 && c->src.ready() && c->src.plane_sharded()) {  // the rank's brick planes of the (windowed) source index
+  if (c->ex.world == 1 && c->src.ready() && c->src.windowed()) c->src.widen(c->stream);
+  if (c->ex.world > 1 && c->src.ready() && c->src.plane_sharded()) {  // the rank's brick planes of the (windowed) source index
     c->shard_lo = c->src.shard_lo();
     c->shard_hi = c->src.shard_hi();
   } else {
     const int64_t n = c->src.ready() ? c->src.n_indexed() : 0;
-    c->shard_lo = (int)(n * c->rank / c->world);
-    c->shard_hi = (int)(n * (c->rank + 1) / c->world);
+    c->shard_lo = (int)(n * c->ex.rank / c->ex.world);
+    c->shard_hi = (int)(n * (c->ex.rank + 1) / c->ex.world);
   }
   if (c->shard_lo != lo || c->shard_hi != hi) {
     c->cov_ready = false;
@@ -401,8 +289,8 @@ void update_shard(gicpb_ctx* c) {
 
 // Target covariances are needed in full on every rank, but each is a function of the target cloud alone: every rank
 // computes one contiguous chunk of the (identically sorted) target (start_target_cov, on `knn_stream`) and the chunks
-// are all-gathered in place (finish_covariances, on the context's stream).
-int target_chunk(const gicpb_ctx* c) { return (c->tgt.n_indexed() + c->world - 1) / c->world; }
+// are all-gathered in place (Exchange::gather_send there, gather_recv in finish_covariances, on the context's stream).
+int target_chunk(const gicpb_ctx* c) { return (c->tgt.n_indexed() + c->ex.world - 1) / c->ex.world; }
 
 void check_k(const gicpb_ctx* c) {
   const int k = c->prm.k_correspondences;
@@ -413,18 +301,13 @@ void start_target_cov(gicpb_ctx* c, cudaStream_t knn_stream) {
   const int k = c->prm.k_correspondences;
   const int nt = c->tgt.n_indexed();
   const int chunk = target_chunk(c);
-  const int t_lo = std::min(nt, c->rank * chunk), t_hi = std::min(nt, t_lo + chunk);
-  c->n_tgt.reserve(3 * (size_t)chunk * c->world);
+  const int t_lo = std::min(nt, c->ex.rank * chunk), t_hi = std::min(nt, t_lo + chunk);
+  c->n_tgt.reserve(3 * (size_t)chunk * c->ex.world);
   const FarWork fw = far_work(c, chunk);
   launch_knn_covariances(c->tgt.view(), t_lo, t_hi, k, c->n_tgt.get() + 3 * (size_t)t_lo, nullptr, nullptr, fw, knn_stream);
-  c->tgt_normals_gathered = false;
-  if (c->world > 1 && !c->local && knn_stream != c->stream) {
-    // gicpb_set_clouds: the chunks are exchanged on the second stream too, beside the source's index build (a chain of short
-    // kernels that leaves the links and most of the SMs idle), not in front of the source's covariance pass
-    check_nccl(c, c->nccl->AllGather(c->n_tgt.get() + 3 * (size_t)c->rank * chunk, c->n_tgt.get(), 3 * (size_t)chunk,
-                                     kNcclFloat64, c->comm, knn_stream), "ncclAllGather");
-    c->tgt_normals_gathered = true;
-  }
+  // with NCCL, gicpb_set_clouds exchanges the chunks on the second stream too, beside the source's index build (a chain of
+  // short kernels that leaves the links and most of the SMs idle), not in front of the source's covariance pass
+  c->ex.gather_send(c->n_tgt.get(), 3 * sizeof(double) * chunk, knn_stream);
 }
 
 // the rest, on the context's stream (which must already be ordered after start_target_cov's kernels)
@@ -435,21 +318,8 @@ void finish_covariances(gicpb_ctx* c) {
   const int chunk = target_chunk(c);
   c->n_src.reserve(3 * (size_t)std::max(ns, 1));
   const FarWork fw = far_work(c, std::max(chunk, ns));
-  if (c->world > 1 && c->local) {
-    // in-process group: every rank's chunk is complete and its buffer in place, then the other chunks come over NVLink
-    GICPB_CUDA(cudaStreamSynchronize(c->stream));
-    c->local->barrier();
-    for (int r = 0; r < c->world; ++r) {
-      if (r == c->rank) continue;
-      const gicpb_ctx* o = c->local->members[(size_t)r];
-      GICPB_CUDA(cudaMemcpyPeerAsync(c->n_tgt.get() + 3 * (size_t)r * chunk, c->device, o->n_tgt.get() + 3 * (size_t)r * chunk,
-                                     o->device, 3 * (size_t)chunk * sizeof(double), c->stream));
-    }
-  } else if (c->world > 1 && !c->tgt_normals_gathered) {
-    check_nccl(c, c->nccl->AllGather(c->n_tgt.get() + 3 * (size_t)c->rank * chunk, c->n_tgt.get(), 3 * (size_t)chunk,
-                                     kNcclFloat64, c->comm, c->stream), "ncclAllGather");
-  }
-  c->tgt_normals_gathered = false;
+  c->ex.gather_recv(c->n_tgt.get(), 3 * sizeof(double) * chunk, 3 * sizeof(double) * c->tgt.n_indexed(), c->stream,
+                    [c](int r) { return c->group->ctx[(size_t)r]->n_tgt.get(); });
   const GridIndex::KnnWindow win = c->src.knn_window();
   unsigned* violations = c->far_counter.get() + 2;  // far_work() reserved 4 words; [0..1] belong to the far hand-over
   if (win.axis >= 0) {
@@ -461,7 +331,7 @@ void finish_covariances(gicpb_ctx* c) {
     launch_knn_covariances(c->src.view(), c->shard_lo, c->shard_hi, k, c->n_src.get(), nullptr, nullptr, fw, c->stream);
   }
   GICPB_CUDA(cudaStreamSynchronize(c->stream));
-  if (c->world > 1 && c->local) c->local->barrier();  // nobody touches its n_tgt again before every copy out of it is done
+  c->ex.barrier(c->stream);  // nobody touches its n_tgt again before every copy out of it is done
   if (win.axis >= 0 && c->h_far[2] != 0u) {
     // some neighbourhoods of this rank's shard reach beyond the halo of its window (a sparse region): index the whole source
     // after all - the shard stays the same set of points - and take the covariances from that
@@ -528,7 +398,7 @@ void run_correspondences(gicpb_ctx* c, const float* T16, bool first, int near_ri
     const int n = c->shard_hi - c->shard_lo;
     launch_moments(c->src.sorted_points(), c->shard_lo, n, c->pair_tgt.get(), c->maha.get(), fp32, T,
                    c->mom_partials.get(), c->ticket.get(), c->d_mom.get(), moments_grid_blocks(n, c->num_sms), c->stream);
-    all_reduce_sum(c, c->d_mom.get(), kMomentSums);
+    c->ex.all_reduce_sum(c->d_mom.get(), kMomentSums, c->stream);
     GICPB_CUDA(cudaMemcpyAsync(c->h_mom, c->d_mom.get(), kMomentSums * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     std::memcpy(c->mom_T0, T16, sizeof(c->mom_T0));
   }
@@ -569,8 +439,8 @@ void cost_from_moments(gicpb_ctx* c, const double* x, double* sums) {
 
 // ---- persistent evaluation session (one per inner solve) --------------------------------------------------------------------
 bool cost_session_wanted(const gicpb_ctx* c) {
-  return c->prm.cost_persistent != 0 && c->prm.cost_moments == 0 && (c->world == 1 || c->peer_ready) && c->h_cmd != nullptr &&
-         c->shard_hi > c->shard_lo;
+  return c->prm.cost_persistent != 0 && c->prm.cost_moments == 0 && (c->ex.world == 1 || c->ex.fused_sum()) &&
+         c->h_cmd != nullptr && c->shard_hi > c->shard_lo;
 }
 
 void cost_session_begin(gicpb_ctx* c) {
@@ -579,10 +449,9 @@ void cost_session_begin(gicpb_ctx* c) {
   c->cost_epoch = (c->cost_epoch % 4094u) + 1u;
   c->cost_count = 0;
   c->d_cmd.reserve(1);
-  const bool fused = c->world > 1 && c->peer_ready;
   launch_cost_persistent(c->src.sorted_points(), c->shard_lo, c->shard_hi - c->shard_lo, c->pair_tgt.get(), c->maha.get(),
                          c->pairs_fp32, c->h_cmd_dev + (c->cost_epoch & 1u), c->d_cmd.get(), c->cost_epoch, c->partials.get(), c->ticket.get(),
-                         c->h_sums_dev, fused ? &c->peer : nullptr, c->cost_idle_ns, cost_persistent_blocks(c->num_sms),
+                         c->h_sums_dev, c->ex.fused_sum(), c->cost_idle_ns, cost_persistent_blocks(c->num_sms),
                          c->smem_optin, c->stream, &c->cost_shape);
   c->cost_live = true;
 }
@@ -632,10 +501,10 @@ void run_cost(gicpb_ctx* c, const double* x, double* sums) {
   const Rigid T = rigid_from_rowmajor(T16);
   const int n = c->shard_hi - c->shard_lo;
   const int blocks = cost_grid_blocks(n, c->num_sms);
-  const bool fused = c->world > 1 && c->peer_ready;
-  double* out = (c->world > 1 && !fused) ? c->d_sums.get() : c->h_sums_dev;
+  const PeerReduce* fused = c->ex.fused_sum();
+  double* out = (c->ex.world > 1 && !fused) ? c->d_sums.get() : c->h_sums_dev;
   if (fused) {
-    if (++c->peer.seq == 0u) c->peer.seq = 1u;
+    if (++c->ex.peer.seq == 0u) c->ex.peer.seq = 1u;
   }
   // the sums land in mapped host memory: the host polls the stamp the kernel stores after them (no driver call between
   // the kernel's last store and the optimiser's next step); the NCCL path still synchronises the stream
@@ -656,10 +525,10 @@ void run_cost(gicpb_ctx* c, const double* x, double* sums) {
     }
   }
   if (session)
-    cost_session_send(c, kCostOpEval, T16, stamp, c->peer.seq);
+    cost_session_send(c, kCostOpEval, T16, stamp, c->ex.peer.seq);
   else
     launch_cost(c->src.sorted_points(), c->shard_lo, n, c->pair_tgt.get(), c->maha.get(), c->pairs_fp32, T,
-                c->partials.get(), c->ticket.get(), out, blocks, c->stream, fused ? &c->peer : nullptr, stamp);
+                c->partials.get(), c->ticket.get(), out, blocks, c->stream, fused, stamp);
   if (polled) {
     // 28 self-validating words (kernels.hpp launch_cost): every one must show this evaluation's stamp
     const volatile unsigned long long* words = reinterpret_cast<const volatile unsigned long long*>(c->h_sums + kCostOutWords);
@@ -684,7 +553,7 @@ void run_cost(gicpb_ctx* c, const double* x, double* sums) {
             // the command: launch it again and repeat the command
             ++relaunches;
             cost_session_begin(c);
-            cost_session_send(c, kCostOpEval, T16, stamp, c->peer.seq);
+            cost_session_send(c, kCostOpEval, T16, stamp, c->ex.peer.seq);
             continue;
           }
           throw CudaError("cost kernel finished without publishing its sums");
@@ -698,16 +567,13 @@ void run_cost(gicpb_ctx* c, const double* x, double* sums) {
       std::memcpy(&c->h_sums[i], &bits, sizeof(double));
     }
   } else {
-    all_reduce_sum(c, c->d_sums.get(), kCostSums);
+    c->ex.all_reduce_sum(c->d_sums.get(), kCostSums, c->stream);
     GICPB_CUDA(cudaMemcpyAsync(c->h_sums, c->d_sums.get(), kCostSums * sizeof(double), cudaMemcpyDeviceToHost,
                                c->stream));
     GICPB_CUDA(cudaStreamSynchronize(c->stream));
   }
   for (int i = 0; i < kCostSums; ++i) sums[i] = c->h_sums[i];
-  if (fused && std::isnan(sums[13])) {
-    c->peer_ready = false;  // the slot flags are out of step from here on: this context goes back to ncclAllReduce
-    throw NcclError("peer-memory reduction timed out: a rank did not launch this evaluation (GICPB_PEER_TIMEOUT_MS)");
-  }
+  if (fused && std::isnan(sums[13])) c->ex.fused_sum_timed_out();
   ++c->cost_evals;
 }
 
@@ -864,32 +730,14 @@ void check_cloud_args(const void* p, int64_t n, int64_t stride) {
 }
 
 // Sharded upload (world > 1, host clouds): every rank is given the same clouds, so each uploads only its 1 / world of the
-// rows (packed xyz, 12 bytes per point) and the slices are exchanged between the GPUs - one in-place ncclAllGather, or peer
-// copies inside a gicpb_group - instead of every rank pulling both whole clouds through its host.  GICPB_SHARD_UPLOAD=0: off.
+// rows (packed xyz, 12 bytes per point) and the slices are all-gathered between the GPUs (Exchange) instead of every rank
+// pulling both whole clouds through its host.  GICPB_SHARD_UPLOAD=0: off.
 bool shard_uploads(const gicpb_ctx* c) {
   static const bool enabled = [] {
     const char* e = std::getenv("GICPB_SHARD_UPLOAD");
     return !(e && *e == '0');
   }();
-  return enabled && c->world > 1 && (c->local != nullptr || c->comm != nullptr);
-}
-
-// in-process group: the other members' slices are copied over from their staging buffers when the cloud is set
-void gather_slices(gicpb_ctx* c, int which) {
-  gicpb_ctx::Prefetch& p = c->prefetch[which];
-  const size_t chunk_bytes = (size_t)p.chunk_rows * 12;
-  GICPB_CUDA(cudaStreamSynchronize(c->stream));  // this rank's slice is in place (the stream waits for the copy stream)
-  c->local->barrier();
-  for (int r = 0; r < c->world; ++r) {
-    if (r == c->rank) continue;
-    const int64_t lo = std::min<int64_t>(p.n, (int64_t)r * p.chunk_rows), hi = std::min<int64_t>(p.n, lo + p.chunk_rows);
-    if (hi <= lo) continue;
-    const gicpb_ctx* o = c->local->members[(size_t)r];
-    GICPB_CUDA(cudaMemcpyPeerAsync(p.dev + (size_t)r * chunk_bytes, c->device, o->prefetch[which].dev + (size_t)r * chunk_bytes,
-                                   o->device, (size_t)(hi - lo) * 12, c->stream));
-  }
-  GICPB_CUDA(cudaStreamSynchronize(c->stream));
-  c->local->barrier();  // every rank has what it needs from the others' staging buffers
+  return enabled && c->ex.may_shard_uploads();
 }
 
 // starts the upload of a host cloud on the copy stream (gicpb_prefetch_cloud)
@@ -909,9 +757,9 @@ void do_prefetch(gicpb_ctx* c, int which, const void* xyz, int64_t n, int64_t st
   const unsigned char* src = static_cast<const unsigned char*>(xyz);
   p.sharded = shard_uploads(c);
   if (p.sharded) {
-    p.chunk_rows = (n + c->world - 1) / c->world;
-    const int64_t lo = std::min<int64_t>(n, (int64_t)c->rank * p.chunk_rows), hi = std::min<int64_t>(n, lo + p.chunk_rows);
-    p.dev = stage((size_t)p.chunk_rows * c->world * 12);
+    p.chunk_rows = (n + c->ex.world - 1) / c->ex.world;
+    const int64_t lo = std::min<int64_t>(n, (int64_t)c->ex.rank * p.chunk_rows), hi = std::min<int64_t>(n, lo + p.chunk_rows);
+    p.dev = stage((size_t)p.chunk_rows * c->ex.world * 12);
     p.dev_stride = 12;
     if (hi > lo) {
       if (stride == 12 && !HostStager::wants(src + lo * stride, hi - lo, stride))
@@ -930,12 +778,9 @@ void do_prefetch(gicpb_ctx* c, int which, const void* xyz, int64_t n, int64_t st
       GICPB_CUDA(cudaMemcpyAsync(p.dev, xyz, (size_t)(n - 1) * stride + 12, cudaMemcpyHostToDevice, c->copy_stream));
     }
   }
-  if (p.sharded && !c->local) {
-    // one process per GPU: the slices are exchanged on the copy stream as soon as this rank's has arrived - for the source
-    // that is WHILE the target is indexed on the compute stream, not in front of the source's own index build
-    check_nccl(c, c->nccl->AllGather(p.dev + (size_t)c->rank * (size_t)p.chunk_rows * 12, p.dev, (size_t)p.chunk_rows * 12,
-                                     /*ncclInt8*/ 0, c->comm, c->copy_stream), "ncclAllGather");
-  }
+  // with NCCL the slices are exchanged on the copy stream as soon as this rank's has arrived - for the source that is WHILE
+  // the target is indexed on the compute stream, not in front of the source's own index build
+  if (p.sharded) c->ex.gather_send(p.dev, (size_t)p.chunk_rows * 12, c->copy_stream);
   GICPB_CUDA(cudaEventRecord(p.done, c->copy_stream));
   p.host = xyz;
   p.n = n;
@@ -955,7 +800,11 @@ bool take_prefetch(gicpb_ctx* c, int which, const void* xyz, int64_t n, int64_t 
   if (!p.pending) return false;
   p.pending = false;
   GICPB_CUDA(cudaStreamWaitEvent(c->stream, p.done, 0));
-  if (p.sharded && c->local) gather_slices(c, which);
+  if (p.sharded) {  // a group's members copy the other slices from each other's staging buffers here
+    c->ex.gather_recv(p.dev, (size_t)p.chunk_rows * 12, (size_t)p.n * 12, c->stream,
+                      [c, which](int r) { return c->group->ctx[(size_t)r]->prefetch[which].dev; });
+    c->ex.barrier(c->stream);
+  }
   return true;
 }
 
@@ -1034,19 +883,6 @@ int64_t compute_normals(gicpb_ctx* c, int which, double radius, int64_t* total_p
 
 }  // namespace
 
-// ---- one process, several GPUs (include/gicp_b200.h "gicpb_group") ------------------------------------------------------
-// The reference's consumer builds its GICPAlignment inside ONE process (reference src/LeicaStateMachine.cpp:138-171), so the
-// multi-GPU path must be reachable without a launcher: a group owns one context per device, every group call runs the same
-// per-rank call on all of them from one host thread per GPU (exactly what the ranks of a torchrun job do, optimisers in lock
-// step), and the collectives stay inside the process: target covariances by peer copies, the 14 cost sums fused into the cost
-// kernel over peer memory (kernels.hpp PeerReduce) when every pair of devices can map each other, else through the host.
-struct gicpb_group {
-  LocalGroup lg;
-  std::vector<gicpb_ctx*> ctx;
-  std::string err;
-  bool fused = false;
-};
-
 namespace {
 
 template <typename F>
@@ -1060,8 +896,8 @@ int group_run(gicpb_group* g, F fn) {  // fn(rank, ctx) -> status, on one thread
   bool all_ready = true;
   for (int r = 0; r < n; ++r) {
     gicpb_ctx* c = g->ctx[(size_t)r];
-    c->rank = r;
-    c->world = n;
+    c->ex.rank = r;
+    c->ex.world = n;
     update_shard(c);
     all_ready = all_ready && c->cov_ready;
   }
@@ -1074,11 +910,11 @@ int group_run(gicpb_group* g, F fn) {  // fn(rank, ctx) -> status, on one thread
     // a member is rank r of n only while a group call runs on all members at once; used on its own (gicpb_group_ctx) it is
     // a plain single-GPU context, so that nothing it does waits for the other members
     gicpb_ctx* c = g->ctx[(size_t)r];
-    c->rank = r;
-    c->world = n;
+    c->ex.rank = r;
+    c->ex.world = n;
     rc[(size_t)r] = fn(r, c);
-    c->rank = 0;
-    c->world = 1;
+    c->ex.rank = 0;
+    c->ex.world = 1;
     if (rc[(size_t)r] != GICPB_OK) g->lg.fail();  // the others must not wait for this rank at a barrier
   };
   std::vector<std::thread> th;
@@ -1140,8 +976,8 @@ unsigned long long group_difference_rank(gicpb_ctx* c, const void* input, int64_
       sub_dev = true;
     }
     // 2. the window of the subtract's brick planes
-    c->sub.build(sub_p, n_sub, sub_stride, sub_dev, c->prm.cell_size, c->prm.points_per_cell, c->stream, &c->stager, c->rank,
-                 c->world, std::isfinite(radius) ? radius : INFINITY);
+    c->sub.build(sub_p, n_sub, sub_stride, sub_dev, c->prm.cell_size, c->prm.points_per_cell, c->stream, &c->stager, c->ex.rank,
+                 c->ex.world, std::isfinite(radius) ? radius : INFINITY);
     if (take_prefetch(c, 3, input, n, input_stride, 0)) {
       d_in = c->prefetch[3].dev;
       input_stride = c->prefetch[3].dev_stride;
@@ -1156,7 +992,7 @@ unsigned long long group_difference_rank(gicpb_ctx* c, const void* input, int64_
       }
     throw;
   }
-  const int64_t lo = n * c->rank / c->world, hi = n * (c->rank + 1) / c->world, len = hi - lo;
+  const int64_t lo = n * c->ex.rank / c->ex.world, hi = n * (c->ex.rank + 1) / c->ex.world, len = hi - lo;
   const bool routed = c->sub.plane_sharded();
   c->keep_full.reserve((size_t)n);
   GICPB_CUDA(cudaMemsetAsync(c->keep_full.get(), 0, (size_t)n, c->stream));
@@ -1180,22 +1016,19 @@ unsigned long long group_difference_rank(gicpb_ctx* c, const void* input, int64_
   unsigned long long kept = 0;
   GICPB_CUDA(cudaMemcpyAsync(&kept, c->counter.get(), sizeof(kept), cudaMemcpyDeviceToHost, c->stream));
   GICPB_CUDA(cudaStreamSynchronize(c->stream));
-  // 4. ownership partitions the finite rows: the mask of [lo, hi) is the OR of every member's keep bytes there
-  c->local->barrier();  // every member's keep bytes are complete
+  // 4. ownership partitions the finite rows: the mask of [lo, hi) is the OR of every member's keep bytes there, fetched once
+  // every member's are complete
+  const bool merge = routed && len > 0;
+  if (merge) c->keep_parts.reserve((size_t)(c->ex.world * len));
+  c->ex.fetch_all(c->keep_parts.get(), (size_t)lo, merge ? (size_t)len : 0, c->stream,
+                  [c](int r) { return c->group->ctx[(size_t)r]->keep_full.get(); });
   const unsigned char* slice = c->keep_full.get() + lo;
-  if (routed && len > 0) {
-    c->keep_parts.reserve((size_t)(c->world * len));
-    for (int r = 0; r < c->world; ++r) {
-      const gicpb_ctx* o = c->local->members[(size_t)r];
-      GICPB_CUDA(cudaMemcpyPeerAsync(c->keep_parts.get() + r * len, c->device, o->keep_full.get() + lo, o->device, (size_t)len,
-                                     c->stream));
-    }
+  if (merge) {
     c->io_b.reserve((size_t)len);
-    or_parts(c->keep_parts.get(), c->world, len, c->io_b.get(), c->stream);
+    or_parts(c->keep_parts.get(), c->ex.world, len, c->io_b.get(), c->stream);
     slice = c->io_b.get();
   }
-  GICPB_CUDA(cudaStreamSynchronize(c->stream));
-  c->local->barrier();  // nobody reads another member's keep bytes any more
+  c->ex.barrier(c->stream);  // nobody reads another member's keep bytes any more
   if (len > 0) download_bytes(c, mask + lo, slice, (size_t)len);
   return kept;
 }
@@ -1289,16 +1122,11 @@ int gicpb_create(int device, gicpb_ctx** out) {
 void gicpb_destroy(gicpb_ctx* c) {
   if (!c) return;
   DeviceGuard guard(c->device);
-  if (c->comm && c->nccl) c->nccl->CommDestroy(c->comm);
   cost_session_end(c);
   if (c->stream) cudaStreamSynchronize(c->stream);
   if (c->h_sums) cudaFreeHost(c->h_sums);
   if (c->h_cmd) cudaFreeHost(c->h_cmd);
   if (c->h_mom) cudaFreeHost(c->h_mom);
-  if (c->peer.world > 1 && c->peer_ipc)
-    for (int r = 0; r < c->peer.world; ++r)
-      if (r != c->rank && c->peer.peers[r]) cudaIpcCloseMemHandle(c->peer.peers[r]);
-  if (c->peer_own) cudaFree(c->peer_own);
   if (c->h_far) cudaFreeHost(c->h_far);
   for (auto& p : c->prefetch) {
     if (p.pending) cudaEventSynchronize(p.done);
@@ -1335,32 +1163,19 @@ int gicpb_get_params(const gicpb_ctx* c, gicpb_params* p) {
 }
 
 int gicpb_nccl_unique_id(const char* libnccl_path, unsigned char id_out[128]) {
-  std::string err;
-  NcclApi* api = load_nccl(libnccl_path, err);
-  if (!api || !id_out) return GICPB_E_NCCL;
-  NcclApi::unique_id id;
-  if (api->GetUniqueId(&id) != 0) return GICPB_E_NCCL;
-  std::memcpy(id_out, id.internal, 128);
-  return GICPB_OK;
+  return nccl_unique_id(libnccl_path, id_out) ? GICPB_OK : GICPB_E_NCCL;
 }
 
 int gicpb_comm_init(gicpb_ctx* c, const char* libnccl_path, int rank, int world, const unsigned char id[128]) {
   return guarded(c, [&] {
     if (world < 1 || rank < 0 || rank >= world) throw ArgError("bad rank / world");
     if (world == 1) {
-      c->rank = 0;
-      c->world = 1;
+      c->ex.rank = 0;
+      c->ex.world = 1;
       return;
     }
     if (!id) throw ArgError("null NCCL unique id");
-    std::string err;
-    c->nccl = load_nccl(libnccl_path, err);
-    if (!c->nccl) throw NcclError(err);
-    NcclApi::unique_id uid;
-    std::memcpy(uid.internal, id, 128);
-    check_nccl(c, c->nccl->CommInitRank(&c->comm, world, uid, rank), "ncclCommInitRank");
-    c->rank = rank;
-    c->world = world;
+    c->ex.init_nccl(libnccl_path, rank, world, id);
     c->cov_ready = false;
     c->pairs_valid = false;
     update_shard(c);
@@ -1371,12 +1186,9 @@ int gicpb_peer_export(gicpb_ctx* c, unsigned char handle_out[64]) {
   return guarded(c, [&] {
     if (!handle_out) throw ArgError("null handle");
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
-    if (!c->peer_own) {
-      GICPB_CUDA(cudaMalloc(&c->peer_own, sizeof(PeerSlots)));
-      GICPB_CUDA(cudaMemset(c->peer_own, 0, sizeof(PeerSlots)));
-    }
+    c->ex.alloc_peer_slots();
     cudaIpcMemHandle_t h;
-    GICPB_CUDA(cudaIpcGetMemHandle(&h, c->peer_own));
+    GICPB_CUDA(cudaIpcGetMemHandle(&h, c->ex.peer_own));
     std::memcpy(handle_out, &h, 64);
   });
 }
@@ -1384,39 +1196,31 @@ int gicpb_peer_export(gicpb_ctx* c, unsigned char handle_out[64]) {
 int gicpb_peer_import(gicpb_ctx* c, const unsigned char* handles, int world) {
   return guarded(c, [&] {
     if (!handles) throw ArgError("null handles");
-    if (world != c->world || world < 2 || world > kMaxPeers) throw ArgError("world must match gicpb_comm_init (2..16)");
-    if (!c->peer_own) throw StateError("gicpb_peer_export must be called first");
-    c->peer_ready = false;
+    if (world != c->ex.world || world < 2 || world > kMaxPeers) throw ArgError("world must match gicpb_comm_init (2..16)");
+    if (!c->ex.peer_own) throw StateError("gicpb_peer_export must be called first");
+    c->ex.peer_ready = false;
     // seq restarts at 0 below: the flag words of an earlier import must not look like evaluations already done
     GICPB_CUDA(cudaStreamSynchronize(c->stream));
-    GICPB_CUDA(cudaMemset(c->peer_own, 0, sizeof(PeerSlots)));
+    GICPB_CUDA(cudaMemset(c->ex.peer_own, 0, sizeof(PeerSlots)));
+    PeerSlots* peers[kMaxPeers] = {};
     for (int r = 0; r < world; ++r) {
-      if (r == c->rank) {
-        c->peer.peers[r] = c->peer_own;
+      if (r == c->ex.rank) {
+        peers[r] = c->ex.peer_own;
         continue;
       }
       cudaIpcMemHandle_t h;
       std::memcpy(&h, handles + 64 * (size_t)r, 64);
       void* p = nullptr;
       GICPB_CUDA(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
-      c->peer.peers[r] = static_cast<PeerSlots*>(p);
+      peers[r] = static_cast<PeerSlots*>(p);
     }
-    c->peer.rank = c->rank;
-    c->peer.world = world;
-    c->peer.seq = 0u;
-    c->peer_ipc = true;
-    {
-      const char* env = std::getenv("GICPB_PEER_TIMEOUT_MS");
-      const double ms = env && *env ? std::atof(env) : 30000.0;
-      c->peer.timeout_ns = (unsigned long long)(std::max(ms, 1.0) * 1e6);
-    }
-    c->peer_ready = true;
+    c->ex.arm_fused_sum(c->ex.rank, world, peers, true);
   });
 }
 
 int gicpb_peer_disable(gicpb_ctx* c) {
   if (!c) return GICPB_E_BADARG;
-  c->peer_ready = false;  // back to ncclAllReduce; mapped handles stay open until gicpb_destroy
+  c->ex.peer_ready = false;  // back to all_reduce_sum; mapped handles stay open until gicpb_destroy
   return GICPB_OK;
 }
 
@@ -1431,8 +1235,8 @@ int gicpb_shard_info(gicpb_ctx* c, int64_t* lo, int64_t* hi, int64_t* n_indexed_
 
 int gicpb_comm_rank(const gicpb_ctx* c, int* rank, int* world) {
   if (!c) return GICPB_E_BADARG;
-  if (rank) *rank = c->rank;
-  if (world) *world = c->world;
+  if (rank) *rank = c->ex.rank;
+  if (world) *world = c->ex.world;
   return GICPB_OK;
 }
 
@@ -1468,8 +1272,8 @@ int gicpb_set_source(gicpb_ctx* c, const void* xyz, int64_t n, int64_t stride, i
       stride = c->prefetch[1].dev_stride;
       on_device = 1;
     }
-    c->src.build(xyz, n, stride, on_device != 0, c->prm.cell_size, c->prm.points_per_cell, c->stream, &c->stager, c->rank,
-                 c->world);
+    c->src.build(xyz, n, stride, on_device != 0, c->prm.cell_size, c->prm.points_per_cell, c->stream, &c->stager, c->ex.rank,
+                 c->ex.world);
     update_shard(c);
   });
 }
@@ -1506,7 +1310,7 @@ int gicpb_set_clouds(gicpb_ctx* c, const void* target, int64_t n_target, int64_t
         s_dev = 1;
       }
       c->src.build(source, n_source, source_stride, s_dev != 0, c->prm.cell_size, c->prm.points_per_cell, c->stream, &c->stager,
-                   c->rank, c->world);
+                   c->ex.rank, c->ex.world);
     } catch (...) {
       if (overlap) cudaStreamSynchronize(c->aux_stream);  // nothing may still be running on the target when we leave
       throw;
@@ -1545,7 +1349,7 @@ int gicpb_fitness(gicpb_ctx* c, const float transform[16], double max_range, dou
     const int* seed = (c->prm.use_previous_match != 0 && c->pairs_valid) ? c->pair_pos.get() : nullptr;
     launch_fitness(c->tgt.view(), c->src.sorted_points(), c->shard_lo, c->shard_hi, T, max_range, seed, partials,
                    c->d_sums.get(), far_work(c, c->shard_hi - c->shard_lo), c->stream);
-    all_reduce_sum(c, c->d_sums.get(), 2);
+    c->ex.all_reduce_sum(c->d_sums.get(), 2, c->stream);
     GICPB_CUDA(cudaMemcpyAsync(c->h_sums, c->d_sums.get(), 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     GICPB_CUDA(cudaStreamSynchronize(c->stream));
     *score = c->h_sums[1] > 0 ? c->h_sums[0] / c->h_sums[1] : std::numeric_limits<double>::max();
@@ -2145,8 +1949,7 @@ int gicpb_group_create(const int* devices, int n_devices, gicpb_group** out) {
     *out = g.release();
     return GICPB_OK;
   }
-  g->lg.world = n_devices;
-  g->lg.members = g->ctx;
+  g->lg.devices.assign(devices, devices + n_devices);
   g->lg.slots.assign(80 * (size_t)n_devices, 0.0);
   // The fused sum makes each rank's cost kernel wait for the other ranks' kernels: only sound when every rank has a GPU of
   // its own (two such kernels on one GPU may never run at the same time) and every pair can map each other's memory.
@@ -2163,7 +1966,8 @@ int gicpb_group_create(const int* devices, int n_devices, gicpb_group** out) {
     for (int r = 0; r < n_devices; ++r) {
       gicpb_ctx* c = g->ctx[(size_t)r];
       DeviceGuard guard(c->device);
-      c->local = &g->lg;  // rank / world are set for the duration of each group call (group_run)
+      c->ex.local = &g->lg;  // rank / world are set for the duration of each group call (group_run)
+      c->group = g.get();
       if (!fused) continue;
       for (int b = 0; b < n_devices; ++b) {
         if (b == r) continue;
@@ -2171,22 +1975,12 @@ int gicpb_group_create(const int* devices, int n_devices, gicpb_group** out) {
         if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) GICPB_CUDA(e);
         (void)cudaGetLastError();
       }
-      GICPB_CUDA(cudaMalloc(&c->peer_own, sizeof(PeerSlots)));
-      GICPB_CUDA(cudaMemset(c->peer_own, 0, sizeof(PeerSlots)));
+      c->ex.alloc_peer_slots();
     }
     if (fused) {
-      const char* env = std::getenv("GICPB_PEER_TIMEOUT_MS");
-      const double ms = env && *env ? std::atof(env) : 30000.0;
-      for (int r = 0; r < n_devices; ++r) {
-        gicpb_ctx* c = g->ctx[(size_t)r];
-        for (int b = 0; b < n_devices; ++b) c->peer.peers[b] = g->ctx[(size_t)b]->peer_own;  // plain device pointers (UVA)
-        c->peer.rank = r;
-        c->peer.world = n_devices;
-        c->peer.seq = 0u;
-        c->peer.timeout_ns = (unsigned long long)(std::max(ms, 1.0) * 1e6);
-        c->peer_ipc = false;
-        c->peer_ready = true;
-      }
+      PeerSlots* peers[kMaxPeers] = {};
+      for (int b = 0; b < n_devices; ++b) peers[b] = g->ctx[(size_t)b]->ex.peer_own;  // plain device pointers (UVA)
+      for (int r = 0; r < n_devices; ++r) g->ctx[(size_t)r]->ex.arm_fused_sum(r, n_devices, peers, false);
     }
   } catch (const std::exception&) {
     cleanup();
@@ -2272,7 +2066,7 @@ int gicpb_group_cloud_difference(gicpb_group* g, const void* input, int64_t n_in
   std::vector<int> rcs(g->ctx.size(), GICPB_OK);
   std::vector<unsigned long long> kept(g->ctx.size(), 0ull);
   const int rc = group_run(g, [&](int r, gicpb_ctx* c) {
-    if (c->world == 1) {  // a group of one device is a plain context
+    if (c->ex.world == 1) {  // a group of one device is a plain context
       int64_t k = 0;
       rcs[(size_t)r] = gicpb_cloud_difference(c, input, n_input, input_stride, subtract, n_subtract, subtract_stride, 0,
                                               sqr_threshold, mask, &k);
